@@ -3,13 +3,17 @@
 + 8x8 range stage R2) on B200, with the HBM roofline of the dominant kernel and the reference CPU encoder timed on
 the same box.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One "step" = one pass of the hot path over one 2048x2048 RGBA synthetic texture (BASELINE.json configs[1]) per GPU,
 inputs resident in HBM.  Inputs rotate over 8 distinct resident images (512 MiB of planes > the 126 MB L2) so every
 step reads cold data.  N > 1: one process per GPU, every rank analyses its own textures (sharded by image, no
 collective on the data path; weak scaling); time = max over ranks.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes the result streams of its last timed step (step K - 1, texture
+(K - 1) mod 8) as DIR/<name>.npy, see dump_outputs().  The textures are seeded, so two builds run with the same arguments
+can be compared output for output.
 """
 from __future__ import annotations
 
@@ -35,20 +39,51 @@ NSLOTS = 8
 METRIC = "encoded megapixels/sec (gradient+range stages)"
 UNIT = "MP/s"
 WORKLOAD = "single synthetic 2048x2048 RGBA texture with alpha holes (alpha bitmap + full tile cascade + R2 range stage) per step"
-
-
-def n_regions(steps):
-    """Timed regions of K steps each in one run of the GPU arm (the mean is reported): a single region of 20 steps lasts
-    about a millisecond, which measures launch jitter rather than the GPU."""
-    return max(1, min(10, 400 // max(1, steps)))
+DUMP_LIMIT = 64 << 20          # bytes --dump-outputs may write in all
 
 
 def base_config(args):
-    """`config` of both arms' lines (identical dictionaries: the driver compares them)."""
+    """`config` of both arms' lines (identical dictionaries, so that lines of the two arms can be compared)."""
     return {"workload": WORKLOAD, "images_per_step_per_gpu": 1, "sharding": "by image, no collective",
             "stages": "MipPrefilter + 7x FittingQuadSmooth + 3x DynamicTileCompressor, results left in HBM",
             "l2": "GPU arm: inputs rotate over 8 distinct resident 64 MiB textures (512 MiB > 126 MB L2), so every step reads cold planes",
-            "timed_regions": f"GPU arm: {n_regions(args.steps)} regions of {args.steps} steps, each bracketed by barrier + synchronize, mean reported"}
+            "timed_regions": f"GPU arm: one region of {args.steps} steps bracketed by barrier + synchronize, after an untimed run of the same region"}
+
+
+def dump_outputs(path, r):
+    """Writes what yk_fetch_all returned for one image (Context.fetch_all) as .npy files: per gradient pass k its bitmap
+    and rgbStream (pass<k>_bitmap, pass<k>_rgb, float32) and [TileDone, bbox] (pass<k>_tiledone_bbox, float64); per colour
+    plane n the R2 streams (r2_idx<n>, r2_type<n>, float32); the alpha stage's bitmap (alpha_bitmap, float32) and
+    [bound, remaining, wrote, chunk bbox] (alpha_bound_remaining_wrote_chunk_bbox, float64, chunk bbox zero when no chunk
+    was written).  stream_lengths (float64) holds the length of every stream in that order; a stream of length zero (an
+    alpha stage that rejects no tile, say) has no file of its own.  Every value is a byte or an int32, so the conversion
+    is exact.  Should the files exceed DUMP_LIMIT, every stream is cut to the same share of its elements, drawn with a
+    fixed seed."""
+    streams, out = {}, {}
+    for k, p in enumerate(r["passes"]):
+        if p is not None:
+            streams[f"pass{k}_bitmap"] = p["bitmap"]
+            streams[f"pass{k}_rgb"] = p["rgb"]
+            out[f"pass{k}_tiledone_bbox"] = np.array([p["tiledone"], *p["bbox"]], np.float64)
+    for n, q in enumerate(r["r2"]):
+        streams[f"r2_idx{n}"] = q["idx"]
+        streams[f"r2_type{n}"] = q["type"]
+    a = r["alpha"]
+    if a:
+        streams["alpha_bitmap"] = a["bitmap"]
+        out["alpha_bound_remaining_wrote_chunk_bbox"] = np.array([*a["bound"], a["remaining"], a["wrote"], *(a["chunk_bbox"] or [0] * 4)], np.float64)
+    out["stream_lengths"] = np.array([v.size for v in streams.values()], np.float64)
+    room = DUMP_LIMIT - sum(v.nbytes for v in out.values())
+    keep = min(1.0, room / (4 * sum(v.size for v in streams.values()) or 1))
+    rng = np.random.default_rng(0)
+    for name, v in streams.items():
+        if v.size and keep < 1.0:      # over the limit: the same fixed, seeded share of every stream, in stream order
+            v = v[np.sort(rng.choice(v.size, int(v.size * keep), replace=False))]
+        if v.size:
+            out[name] = v.astype(np.float32)
+    os.makedirs(path, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(path, name + ".npy"), v)
 
 
 def results_digest(r) -> str:
@@ -394,7 +429,10 @@ def main():
     ap.add_argument("--analysis-ctas", type=int, default=-1, help="CTAs of the persistent analysis kernel in the pipelined region (-1: a quarter of the SMs with 8 streams, half with 2-4, else one per SM)")
     ap.add_argument("--roofline-steps", type=int, default=100, help="launches of the separate pass that times the dominant kernel alone")
     ap.add_argument("--no-prewarm", action="store_true", help="skip the clock-settling loop (profiling runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy (batch workload of the GPU arm)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.workload != "batch"):
+        ap.error("--dump-outputs: only the GPU arm's batch workload")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -477,19 +515,18 @@ def main():
     lib.yk_profile.argtypes = [C.c_void_p, C.c_int]
     lib.yk_profile_read.argtypes = [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_longlong)]
     sampler = ClockSampler(physical_gpu_index(local))
-    launches0 = sum(c.launch_count() for c in ctxs)
     joins = [torch.cuda.Event() for _ in streams]
     sampler.sample()
     sampler.start()
-    NREG = n_regions(args.steps)
-    region_ms = []
-    for reg in range(NREG):
+
+    def region(n):
+        """n steps, timed from their first launch to the end of the last one on any stream; ms of the slowest rank."""
         barrier()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record(stream)                      # every stream starts after ev0 ...
         for st in streams[1:]:
             st.wait_event(ev0)
-        for i in range(args.steps):
+        for i in range(n):
             step(i)
         for st, j in zip(streams[1:], joins[1:]):
             j.record(st)
@@ -502,11 +539,18 @@ def main():
             t = torch.tensor([t_ms], device=f"cuda:{local}", dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             t_ms = float(t.item())
-        region_ms.append(t_ms)
+        return t_ms
+
+    # untimed: the same region once more, so that the timed one is not the first run of the event / stream-wait path
+    # (the first of several regions measured slower than the others)
+    region(args.steps)
+    launches0 = sum(c.launch_count() for c in ctxs)
+    ms = region(args.steps)
+    launches = sum(c.launch_count() for c in ctxs) - launches0
     sampler.stop_flag = True
     sampler.sample()
-    ms = sum(region_ms) / len(region_ms)
-    launches = (sum(c.launch_count() for c in ctxs) - launches0) // NREG
+    last = args.steps - 1                       # the results of the last timed step, before anything else runs on its slot
+    dumped = ctxs[last % NCTX].fetch_all((last // NCTX) % (NSLOTS // NCTX)) if args.dump_outputs and rank == 0 else None
     # informational: the kernels' durations inside a pipelined pass (they overlap each other there).  A pass of its own,
     # after the timed regions: the event pair the library records around every launch is host work and two more stream
     # operations per kernel, and the timed region holds the product's own launches only.
@@ -810,10 +854,12 @@ def main():
                 "config": base_config(args),
                 "run": {"pipelining": f"steps are independent textures, issued round-robin on {NCTX} CUDA streams (contexts); analysis launches of {actas or sms} CTAs on {sms} SMs",
                         "kernels_per_step": "yk_k_analyze (persistent, TMA-staged, range stage fused) + yk_k_owner + yk_k_emit",
-                        "region_ms": [round(x, 4) for x in region_ms]},
+                        "region_ms": round(ms, 4)},
                 "parity_checked": parity_checked,
                 "clocks": sampler.result(), "e2e": e2e, "gpu_launches": int(launches), "roofline": roof, "cpu_baseline": cpu,
                 "with_r1": with_r1, "strips": strips_res, "stages_outside_metric": other}
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     for c in ctxs:
         c.close()
