@@ -237,11 +237,15 @@ static int create_fill(yk_ctx* c) {
     const size_t nbx = (W + 63) / 64, latW = W / 4 + 1, latH = H / 4 + 1;
     c->planeCap = W * H;
     auto up = [](size_t v) { return (v + 255) / 256 * 256; };
-    size_t offStatus[YK_NPASS], off = up(YK_HD_INTS * sizeof(int));
+    // group totals of yk_k_emit (a group: YK_EMIT_THREADS nibble words or range tiles) and their super-groups
+    auto groups = [](size_t n) { return (n + YK_EMIT_THREADS - 1) / YK_EMIT_THREADS; };
+    auto supers = [](size_t g) { return (g + YK_SUPER - 1) / YK_SUPER; };
+    size_t offTot[YK_NPASS], offSup[YK_NPASS], off = up(YK_HD_INTS * sizeof(int));
     for (int p = 0; p < YK_NPASS; p++) {
         const YkPassGeom& g = kGeom[p];
-        offStatus[p] = off;
-        off += up(((W + g.bw - 1) / g.bw) * ((H + g.bh - 1) / g.bh) * sizeof(uint32_t));
+        const size_t nGroups = groups(((W + g.bw - 1) / g.bw) * ((H + g.bh - 1) / g.bh) * (size_t)g.bits / 8);
+        offTot[p] = off; off += up(nGroups * sizeof(uint32_t));
+        offSup[p] = off; off += up(supers(nGroups) * sizeof(uint32_t));
     }
     size_t offNib[YK_NPASS];
     for (int p = 0; p < YK_NPASS; p++) {
@@ -249,7 +253,9 @@ static int create_fill(yk_ctx* c) {
         offNib[p] = off;
         off += up(((W + g.bw - 1) / g.bw) * ((H + g.bh - 1) / g.bh) * (size_t)g.bits / 2 + 16);
     }
-    const size_t offR2 = off; off += up(((W / 8) * (H / 8) / YK_EMIT_THREADS + 2) * sizeof(unsigned long long));
+    const size_t r2Groups = groups((W / 8) * (H / 8));
+    const size_t offR2Tot = off; off += up(r2Groups * sizeof(unsigned long long));
+    const size_t offR2Sup = off; off += up(supers(r2Groups) * sizeof(unsigned long long));
     c->zeroABytes = off;
     const size_t offCell = off; off += up((H / 4 + 1) * nbx * sizeof(uint16_t) + 4);
     const size_t offTouch = off; off += up(latW * latH * sizeof(uint32_t));
@@ -270,9 +276,10 @@ static int create_fill(yk_ctx* c) {
         for (int p = 0; p < maxPlanes; p++) if ((rc = dev_alloc(s, &s.owned[p], W * H))) return rc;
         for (int p = 0; p < maxPlanes; p++) if ((rc = dev_alloc(s, &s.ownedU8[p], ((W + 15) / 16 * 16) * H + 256))) return rc;
         s.d.hdr = (int*)za;
-        for (int p = 0; p < YK_NPASS; p++) s.d.emitStatus[p] = (uint32_t*)(za + offStatus[p]);
+        for (int p = 0; p < YK_NPASS; p++) { s.d.rgbTot[p] = (uint32_t*)(za + offTot[p]); s.d.rgbSup[p] = (uint32_t*)(za + offSup[p]); }
         for (int p = 0; p < YK_NPASS; p++) s.d.emitNib[p] = (uint32_t*)(za + offNib[p]);
-        s.d.r2Status = (unsigned long long*)(za + offR2);
+        s.d.r2Tot = (unsigned long long*)(za + offR2Tot);
+        s.d.r2Sup = (unsigned long long*)(za + offR2Sup);
         s.d.cellMask = (uint16_t*)(za + offCell);
         s.d.touchMap = (uint32_t*)(za + offTouch);
         if ((rc = dev_alloc(s, &s.d.alphaKept, ((H + 15) / 16) * ((W + 15) / 16)))) return rc;
@@ -600,7 +607,7 @@ static int enqueue(yk_ctx* c, int slot0, int nSlots, const YkRun& run, bool doEm
             }
         const int nTiles = (a.d.w / 8) * (a.d.h / 8);
         const int r2Groups = (r2Domain && nTiles > 0) ? (nTiles + YK_EMIT_THREADS - 1) / YK_EMIT_THREADS : 0;
-        if (gradGroups > 0) { YkTimed t(c, 2); yk_launch_owner(c->slotsDev, slot0, nSlots, a.d.latW * a.d.latH, krun, c->stream); c->launches++; }
+        if (gradGroups + r2Groups > 0) { YkTimed t(c, 2); yk_launch_owner(c->slotsDev, slot0, nSlots, a.d.latW * a.d.latH, gradGroups > 0, krun, c->stream); c->launches++; }
         if (gradGroups + r2Groups > 0) { YkTimed t(c, 1); yk_launch_emit(c->slotsDev, slot0, nSlots, gradGroups, r2Groups, krun, c->stream); c->launches++; }
     }
     CK(cudaGetLastError());

@@ -45,30 +45,8 @@ static __device__ __forceinline__ void yk_stv64(unsigned long long* p, unsigned 
 static __device__ __forceinline__ void yk_spin() { __nanosleep(20); }
 #endif
 
-// status word: value << 2 | flag (1 = this unit's own total, 2 = inclusive prefix).  Returns the exclusive prefix of unit u
-// and publishes its inclusive prefix.  All 32 lanes call it with the same arguments.
-static __device__ unsigned yk_lookback32(uint32_t* status, int u, unsigned total) {
-    const int lane = threadIdx.x & 31;
-    if (u == 0) { if (lane == 0) yk_stv(&status[0], (total << 2) | 2u); return 0u; }
-    if (lane == 0) yk_stv(&status[u], (total << 2) | 1u);
-    unsigned base = 0;
-    int look = u - 1;
-    while (look >= 0) {
-        const int idx = look - lane;
-        const unsigned st = idx >= 0 ? yk_ldv(&status[idx]) : 2u;       // before the first unit: inclusive prefix 0
-        const unsigned ready = __ballot_sync(YK_FULL, (st & 3u) != 0u);
-        const unsigned incl = __ballot_sync(YK_FULL, (st & 3u) == 2u);
-        const unsigned need = incl ? ((2u << (__ffs((int)incl) - 1)) - 1u) : YK_FULL;     // lanes up to the nearest inclusive prefix
-        if ((ready & need) != need) { yk_spin(); continue; }
-        base += __reduce_add_sync(YK_FULL, ((need >> lane) & 1u) ? (st >> 2) : 0u);
-        if (incl) break;
-        look -= 32;
-    }
-    if (lane == 0) yk_stv(&status[u], ((base + total) << 2) | 2u);
-    return base;
-}
-
-// same with two counters packed in 64 bits: hi << 32 | lo << 2 | flag
+// status word: hi << 32 | lo << 2 | flag (1 = this unit's own totals, 2 = inclusive prefix).  Returns the exclusive prefix of
+// unit u and publishes its inclusive prefix.  All 32 lanes call it with the same arguments.
 static __device__ unsigned long long yk_lookback64(unsigned long long* status, int u, unsigned hi, unsigned lo) {
     const int lane = threadIdx.x & 31;
     const unsigned long long mine = ((unsigned long long)hi << 32) | ((unsigned long long)lo << 2);

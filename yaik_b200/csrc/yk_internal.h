@@ -27,7 +27,7 @@ enum {
     YK_HD_ALPHA_MINX, YK_HD_ALPHA_MINY, YK_HD_ALPHA_MAXX, YK_HD_ALPHA_MAXY,
     YK_HD_R2_CHUNKS, YK_HD_R2_TILES,        // totals from the scan: 16-byte chunks per plane, coded tiles per plane
     YK_HD_R1_NIB0, YK_HD_R1_NIB1, YK_HD_R1_NIB2, YK_HD_R1_DEF0, YK_HD_R1_DEF1, YK_HD_R1_DEF2,
-    YK_HD_TICKET_EMIT, YK_HD_TICKET_ANALYZE, // work tickets: emission groups in stream order / regions of the persistent analysis kernel
+    YK_HD_TICKET_ANALYZE,          // work ticket: regions of the persistent analysis kernel
     YK_HD_PASS0 = 16,              // YK_NPASS * YK_ST_STRIDE ints
     YK_HD_INTS = YK_HD_PASS0 + YK_NPASS * YK_ST_STRIDE
 };
@@ -38,7 +38,10 @@ enum {
 // made long), 128 x 16 for alpha; out-of-image samples arrive as zeros and are never used unclamped.
 struct alignas(64) YkTmap { unsigned long long opaque[16]; };
 #ifndef YK_EMIT_THREADS
-#define YK_EMIT_THREADS 512    // threads of a yk_k_emit CTA == nibble words / range tiles per look-back group (host and device agree on it)
+#define YK_EMIT_THREADS 512    // threads of a yk_k_emit CTA == nibble words / range tiles per group (host and device agree on it)
+#endif
+#ifndef YK_SUPER
+#define YK_SUPER 32             // groups per super-group: the second level of the group totals
 #endif
 #define YK_UNIT_W 128           // pixels a unit of the analysis kernel is wide (two regions)
 #define YK_RAW_PITCH 132        // samples per row of a staged colour box
@@ -70,12 +73,14 @@ struct alignas(128) YkSlotDev {
     int*      hdr;              // YK_HD_INTS ints
     // ---- gradient results
     uint8_t*  bitmap[YK_NPASS];     // pFillBitMap in the reference's swizzled layout
-    uint32_t* emitStatus[YK_NPASS]; // per swizzle block: decoupled look-back word (rgb bytes << 2 | flag)
+    uint32_t* rgbTot[YK_NPASS];     // per group of YK_EMIT_THREADS nibble words: rgb bytes its tiles emit (added by yk_k_owner)
+    uint32_t* rgbSup[YK_NPASS];     //   the same per super-group of YK_SUPER groups
     uint8_t*  rgb[YK_NPASS];        // rgbStream
     uint8_t*  latRGB;               // [latH][latW][3]  CompressF(Round6(clamped pixel),250) at every lattice point
     uint32_t* emitNib[YK_NPASS];    // per tile in stream order 4 bits: which of TL,TR,BL,BR the tile emits (8 tiles per word)
     // ---- range stage R2 (DynamicTileCompressor)
-    unsigned long long* r2Status;   // per group of YK_EMIT_THREADS tiles (row-major tile order): look-back word (chunks << 32 | codedTiles << 2 | flag)
+    unsigned long long* r2Tot;      // per group of YK_EMIT_THREADS tiles (row-major tile order): chunks << 32 | coded tiles (added by yk_k_owner)
+    unsigned long long* r2Sup;      //   the same per super-group of YK_SUPER groups
     uint8_t*  r2Raw[3];         // [h/8][w/8][64] index bytes of every coded tile at a fixed place (written by the analysis kernel)
     uint32_t* r2RawType[3];     // [h/8][w/8] color0 | minCol << 8 | delta << 16
     uint8_t*  r2Idx[3];         // the streams in the reference's order (gathered by yk_k_emit)
@@ -113,7 +118,7 @@ void yk_launch_fold_touch(const YkSlotDev* slotsDev, int slot0, int nSlots, int 
 // one-thread kernels on a strip's stream: publish / wait for an epoch number in (peer-mapped) halo memory
 void yk_launch_flag_set(unsigned* a, unsigned* b, unsigned value, cudaStream_t st);
 void yk_launch_flag_wait(const unsigned* a, const unsigned* b, unsigned value, cudaStream_t st);
-void yk_launch_owner(const YkSlotDev* slotsDev, int slot0, int nSlots, int nPoints, const YkRun& run, cudaStream_t st);
+void yk_launch_owner(const YkSlotDev* slotsDev, int slot0, int nSlots, int nPoints, bool owners, const YkRun& run, cudaStream_t st);   // owners: resolve corner ownership; run.doR2: count the range tiles
 void yk_launch_emit(const YkSlotDev* slotsDev, int slot0, int nSlots, int gradGroups, int r2Groups, const YkRun& run, cudaStream_t st);
 void yk_launch_state(const YkSlotDev* slotsDev, int slot, int nRegions, int32_t* smoothMap, int32_t* mipmapMask,
                      int32_t* mappedRGB, int32_t* recon0, int32_t* recon1, int32_t* recon2, cudaStream_t st);
