@@ -80,6 +80,20 @@ int  yk_set_image(yk_ctx* ctx, int slot, const int32_t* const* planes, int nPlan
 int  yk_set_upload_format(yk_ctx* ctx, int packedU8);
 /* Same, planes already resident in device memory (borrowed, not copied; row pitch == w). */
 int  yk_set_image_device(yk_ctx* ctx, int slot, const int32_t* const* devPlanes, int nPlanes, int w, int h);
+/* The way in for a decoded image as PNG / JPEG decoders (and Image::LoadPNG before it fills the planes, Image.cpp:200-229)
+ * hold it: interleaved 8-bit samples, `channels` bytes per pixel (3 = R,G,B; 4 = R,G,B,A), rows `rowBytes` apart (>= w *
+ * channels, any value).  nPlanes = 3 or `channels` (4 channels with nPlanes 3: alpha ignored).  The bytes move as they are
+ * (4 or 3 per pixel, no host work) and yk_k_unpack8 splits them into the slot's own packed planes on the device; no byte
+ * past the last pixel, rowBytes * (h - 1) + w * channels, is read.
+ * Host variant: pinned memory (yk_host_alloc) is read by DMA asynchronously and must not change until the next
+ * synchronising call on the context; pageable memory works at the driver's staged rate.
+ * Device variant: read by a kernel on the context's stream; the caller orders its own writes before it (yk_set_stream
+ * or a sync).  Not borrowed: the buffer may be reused once that kernel has run.
+ * Both leave the slot exactly as a packed yk_set_image of the same samples does (so such slots batch with packed uploads).
+ * No sample can be out of range.  YK_ERR_ARG: NULL pointer, channels not 3 / 4, nPlanes not 3 / channels, rowBytes
+ * < w * channels, or w / h as for yk_set_image; YK_ERR_CAPACITY as for yk_set_image. */
+int  yk_set_image_interleaved(yk_ctx* ctx, int slot, const uint8_t* pixels, size_t rowBytes, int channels, int nPlanes, int w, int h);
+int  yk_set_image_interleaved_device(yk_ctx* ctx, int slot, const uint8_t* devPixels, size_t rowBytes, int channels, int nPlanes, int w, int h);
 /* Device pointer of plane `p` of `slot` (so a caller can fill it in place); NULL on error. */
 int32_t* yk_device_plane(yk_ctx* ctx, int slot, int p);
 int  yk_reset_state(yk_ctx* ctx, int slot);
@@ -191,7 +205,7 @@ long long yk_launch_count(yk_ctx* ctx);
 
 /* Per-kernel device time: while enabled, every launch is bracketed by a CUDA event pair on the launching stream;
  * yk_profile_read synchronises, sums the elapsed milliseconds per kernel (0 yk_k_analyze, 1 yk_k_emit, 2 yk_k_owner,
- * 3 yk_k_r1_encode, 4 yk_k_chroma; the other entries are unused) with their launch counts, and clears the record.  Used by bench.py's roofline figure. */
+ * 3 yk_k_r1_encode, 4 yk_k_chroma, 5 yk_k_unpack8; the other entries are unused) with their launch counts, and clears the record.  Used by bench.py's roofline figure. */
 int  yk_profile(yk_ctx* ctx, int enable);
 int  yk_profile_read(yk_ctx* ctx, double ms[8], long long count[8]);
 

@@ -22,6 +22,7 @@ STAGE_ALPHA, STAGE_GRADIENT, STAGE_RANGE1D, STAGE_RANGEDYN, STAGE_RANGEDYN3 = 1,
 EXPORTS = [
     "yk_abi_version", "yk_error_string", "yk_last_cuda_error", "yk_device_count", "yk_create", "yk_destroy",
     "yk_set_stream", "yk_sync", "yk_set_analysis_ctas", "yk_sm_count", "yk_host_alloc", "yk_host_free", "yk_set_image", "yk_set_image_device", "yk_set_upload_format",
+    "yk_set_image_interleaved", "yk_set_image_interleaved_device",
     "yk_device_plane", "yk_reset_state", "yk_reset_states", "yk_analyze", "yk_alpha_reject", "yk_prepare_quad_smooth",
     "yk_gradient_pass", "yk_range1d", "yk_range_dyn", "yk_chroma_prepare", "yk_chroma_plane", "yk_range_dyn_chroma", "yk_download_state", "yk_fetch_all", "yk_result_bytes", "yk_launch_count",
     "yk_profile", "yk_profile_read",
@@ -87,6 +88,8 @@ def load_library(path: str | None = None):
     L.yk_sm_count.argtypes = [C.c_void_p]
     L.yk_set_image.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_int]
     L.yk_set_image_device.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_int]
+    L.yk_set_image_interleaved.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int]
+    L.yk_set_image_interleaved_device.argtypes = L.yk_set_image_interleaved.argtypes
     L.yk_reset_state.argtypes = [C.c_void_p, C.c_int]
     L.yk_set_upload_format.argtypes = [C.c_void_p, C.c_int]
     L.yk_reset_states.argtypes = [C.c_void_p, C.c_int, C.c_int]
@@ -202,6 +205,26 @@ class Context:
         ptrs = (C.c_void_p * c)(*dev_ptrs)
         self.dims[slot] = (c, h, w)
         self._ck(self.L.yk_set_image_device(self.ctx, slot, ptrs, c, w, h), "yk_set_image_device")
+
+    def set_image_interleaved(self, pixels: np.ndarray, n_planes=None, slot=0):
+        """An H x W x C uint8 image (C = 3 RGB or 4 RGBA; the row stride may exceed W * C) from host memory."""
+        if pixels.dtype != np.uint8 or pixels.ndim != 3 or pixels.strides[1:] != (pixels.shape[2], 1):
+            pixels = np.ascontiguousarray(pixels, dtype=np.uint8)
+        h, w, ch = pixels.shape
+        self._keep[slot] = pixels
+        self.set_image_interleaved_ptr(pixels.ctypes.data, pixels.strides[0], ch, n_planes or ch, w, h, slot)
+        self.sync()      # the source array may be pageable numpy memory
+
+    def set_image_interleaved_ptr(self, ptr, row_bytes, channels, n_planes, w, h, slot=0):
+        """Interleaved rows at a host address (pinned from yk_host_alloc: asynchronous until the next synchronising call)."""
+        self.dims[slot] = (n_planes, h, w)
+        self._ck(self.L.yk_set_image_interleaved(self.ctx, slot, C.c_void_p(ptr), row_bytes, channels, n_planes, w, h), "yk_set_image_interleaved")
+
+    def set_image_interleaved_device(self, dev_ptr, row_bytes, channels, n_planes, w, h, slot=0):
+        """Interleaved rows in device memory, read by a kernel on the context's stream (the buffer is not kept)."""
+        self.dims[slot] = (n_planes, h, w)
+        self._ck(self.L.yk_set_image_interleaved_device(self.ctx, slot, C.c_void_p(dev_ptr), row_bytes, channels, n_planes, w, h),
+                 "yk_set_image_interleaved_device")
 
     def device_plane(self, slot, p):
         return self.L.yk_device_plane(self.ctx, slot, p)

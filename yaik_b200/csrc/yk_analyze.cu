@@ -1188,6 +1188,49 @@ yk_k_expand(const YkSlotDev* __restrict__ slots, int slot, int w, int h, int32_t
     for (int p = 0; p < S.nPlanes; p++) if (d[p]) d[p][(size_t)y * w + x] = S.planeU8[p][(size_t)y * S.pitchU8 + x];
 }
 
+// Interleaved 8-bit pixels (C = 3: R,G,B; 4: R,G,B,A; rows rowBytes apart) -> the slot's packed planes (yk_set_image_interleaved).
+// A thread takes 16 pixels of a row: C uint4 loads when the rows are 16-byte aligned and all 16 pixels exist, else byte loads
+// of the 4-pixel units inside the row (w is a multiple of 4), so that nothing past a row's last pixel is read.  One uint4
+// store per plane; the packed row's padding gets zeros, as the host packing writes.
+template <int C> static __device__ __forceinline__ uint32_t yk_unpack_unit(const uint32_t* u, int p) {
+    // C words hold 4 pixels; byte C * i + p is sample p of pixel i
+    uint32_t r = 0;
+#pragma unroll
+    for (int i = 0; i < 4; i++) r |= ((u[(C * i + p) >> 2] >> (8 * ((C * i + p) & 3))) & 255u) << (8 * i);
+    return r;
+}
+template <int C>
+__global__ void __launch_bounds__(256)
+yk_k_unpack8(YkUnpackArgs a) {
+    const int groups = (a.w + 15) >> 4;
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= (long long)groups * a.h) return;
+    const int y = (int)(idx / groups), x0 = (int)(idx - (long long)y * groups) * 16;
+    const uint8_t* row = a.src + (size_t)y * a.rowBytes + (size_t)x0 * C;
+    uint32_t u[4 * C];
+    if (((((uintptr_t)a.src) | a.rowBytes) & 15) == 0 && x0 + 16 <= a.w) {
+#pragma unroll
+        for (int k = 0; k < C; k++) {
+            const uint4 v = reinterpret_cast<const uint4*>(row)[k];
+            u[4 * k] = v.x; u[4 * k + 1] = v.y; u[4 * k + 2] = v.z; u[4 * k + 3] = v.w;
+        }
+    } else {
+#pragma unroll
+        for (int k = 0; k < 4 * C; k++) u[k] = 0;
+#pragma unroll
+        for (int j = 0; j < 4; j++)
+            if (x0 + 4 * j < a.w)
+#pragma unroll
+                for (int b = 0; b < 4 * C; b++) u[C * j + (b >> 2)] |= (uint32_t)row[4 * C * j + b] << (8 * (b & 3));
+    }
+    const size_t o = (size_t)y * a.pitch + x0;
+#pragma unroll
+    for (int p = 0; p < C; p++)
+        if (p < a.nPlanes)
+            *reinterpret_cast<uint4*>(a.dst[p] + o) = make_uint4(yk_unpack_unit<C>(u, p), yk_unpack_unit<C>(u + C, p),
+                                                                 yk_unpack_unit<C>(u + 2 * C, p), yk_unpack_unit<C>(u + 3 * C, p));
+}
+
 // A new launch on a state that already holds claims: every touched lattice point becomes "claimed before" (bit 31).
 __global__ void __launch_bounds__(256)
 yk_k_fold_touch(const YkSlotDev* __restrict__ slots, int slot0, int nWords) {
@@ -1223,6 +1266,12 @@ void yk_launch_analyze(const YkSlotDev* slotsDev, int slot0, int nSlots, int nRe
 void yk_launch_expand(const YkSlotDev* slotsDev, int slot, int nPlanes, int w, int h, int32_t* const* dst, cudaStream_t st) {
     YK_LAUNCH(yk_k_expand, dim3((w + 255) / 256, h), dim3(256), 0, st, slotsDev, slot, w, h, dst[0], dst[1], dst[2], nPlanes > 3 ? dst[3] : (int32_t*)nullptr);
 }
+void yk_launch_unpack8(const YkUnpackArgs& a, int channels, cudaStream_t st) {
+    const long long threads = (long long)((a.w + 15) >> 4) * a.h;
+    const dim3 grid((unsigned)((threads + 255) / 256));
+    if (channels == 4) YK_LAUNCH(yk_k_unpack8<4>, grid, dim3(256), 0, st, a);
+    else YK_LAUNCH(yk_k_unpack8<3>, grid, dim3(256), 0, st, a);
+}
 void yk_launch_fold_touch(const YkSlotDev* slotsDev, int slot0, int nSlots, int nWords, cudaStream_t st) {
     YK_LAUNCH(yk_k_fold_touch, dim3((nWords + 255) / 256, nSlots), dim3(256), 0, st, slotsDev, slot0, nWords);
 }
@@ -1235,6 +1284,8 @@ int yk_preload_analyze() {
     { const cudaError_t e = cudaFuncGetAttributes(&fa, yk_k_analyze); if (e != cudaSuccess) return (int)e; }
     { const cudaError_t e = cudaFuncGetAttributes(&fa, yk_k_analyze_u8); if (e != cudaSuccess) return (int)e; }
     { const cudaError_t e = cudaFuncGetAttributes(&fa, yk_k_expand); if (e != cudaSuccess) return (int)e; }
+    { const cudaError_t e = cudaFuncGetAttributes(&fa, yk_k_unpack8<3>); if (e != cudaSuccess) return (int)e; }
+    { const cudaError_t e = cudaFuncGetAttributes(&fa, yk_k_unpack8<4>); if (e != cudaSuccess) return (int)e; }
     { const cudaError_t e = cudaFuncGetAttributes(&fa, yk_k_fold_touch); if (e != cudaSuccess) return (int)e; }
 #endif
     return 0;

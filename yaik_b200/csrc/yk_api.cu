@@ -104,7 +104,11 @@ struct yk_ctx {
     size_t planeCap = 0;
     // optional per-kernel timing with CUDA events on the launching stream (yk_profile)
     bool profile = false;
-    std::vector<cudaEvent_t> evA[5], evB[5];      // 0 analyze, 1 emit, 2 owner, 3 r1_encode, 4 chroma
+    std::vector<cudaEvent_t> evA[6], evB[6];      // 0 analyze, 1 emit, 2 owner, 3 r1_encode, 4 chroma, 5 unpack8
+    // device copy of the caller's interleaved rows (yk_set_image_interleaved), same row stride; allocated on first use and
+    // grown on demand.  One per context is enough: stream order puts every copy into it after the unpack of the previous one.
+    // Its base is 256-byte aligned, so 16-byte aligned rows take yk_k_unpack8's vector path whatever the caller's base.
+    uint8_t* stage8 = nullptr; size_t stage8Bytes = 0;
 };
 
 struct YkTimed {        // records an event pair around one launch when profiling is on
@@ -320,6 +324,7 @@ extern "C" void yk_destroy(yk_ctx* c) {
     }
     if (c->packer) yk_hostpack_destroy(c->packer);
     cudaFree(c->slotsDev); cudaFree(c->zeroArea);
+    if (c->stage8) cudaFree(c->stage8);
     if (c->lutDev) cudaFree(c->lutDev);
     if (c->rtabDev) cudaFree(c->rtabDev);
     if (c->r7Dev) cudaFree(c->r7Dev);
@@ -360,7 +365,7 @@ extern "C" int yk_profile_read(yk_ctx* c, double ms[8], long long count[8]) {
     CK(cudaSetDevice(c->device));
     CK(cudaStreamSynchronize(c->stream));
     for (int k = 0; k < 8; k++) { ms[k] = 0; count[k] = 0; }
-    for (int k = 0; k < 5; k++) {
+    for (int k = 0; k < 6; k++) {
         for (size_t i = 0; i < c->evA[k].size(); i++) {
             float t = 0;
             if (cudaEventElapsedTime(&t, c->evA[k][i], c->evB[k][i]) == cudaSuccess) { ms[k] += t; count[k]++; }
@@ -423,6 +428,22 @@ extern "C" int yk_set_upload_format(yk_ctx* c, int packedU8) {
     return YK_OK;
 }
 
+// The slot's samples are in its own packed planes (ownedU8, row pitch (w + 15) / 16 * 16, padding zero): the state every
+// stage expects after a packed upload, whichever way the bytes arrived.
+static int use_packed_planes(yk_ctx* c, int slot) {
+    YkSlotHost& s = c->slots[slot];
+    for (int p = 0; p < 4; p++) {
+        s.d.planeU8[p] = p < s.d.nPlanes ? s.ownedU8[p] : nullptr;
+        s.d.plane[p] = p < s.d.nPlanes ? s.owned[p] : nullptr;
+    }
+    s.d.isU8 = 1; s.d.pitchU8 = (s.d.w + 15) / 16 * 16;
+    s.int32Valid = false;
+    s.borrowed = false;
+    const int rc = encode_slot_tmaps(s);
+    if (rc) return rc;
+    return yk_reset_state(c, slot);
+}
+
 extern "C" int yk_set_image(yk_ctx* c, int slot, const int32_t* const* planes, int nPlanes, int w, int h) {
     if (!slot_ok(c, slot) || !planes) return YK_ERR_ARG;
     int rc = configure_slot(c, slot, nPlanes, w, h);
@@ -431,8 +452,7 @@ extern "C" int yk_set_image(yk_ctx* c, int slot, const int32_t* const* planes, i
     CK(cudaSetDevice(c->device));
     for (int p = 0; p < nPlanes; p++) if (!planes[p]) return YK_ERR_ARG;
     unsigned bad = 0;
-    bool packed = c->packedUpload != 0;
-    if (packed) {
+    if (c->packedUpload) {
         // Plane samples are 0..255 on this path: pack them to bytes on the host (threads, range check included) and move a
         // quarter of the bytes over PCIe; yk_k_analyze_u8 stages the packed planes with byte TMA boxes
         const size_t pitch = ((size_t)w + 15) / 16 * 16, planeBytes = pitch * h, need = planeBytes * nPlanes;
@@ -448,26 +468,20 @@ extern "C" int yk_set_image(yk_ctx* c, int slot, const int32_t* const* planes, i
         for (int p = 0; p < nPlanes; p++) {
             bad |= yk_hostpack_plane(c->packer, planes[p], s.stageHost + p * planeBytes, w, h, pitch);
             CK(cudaMemcpyAsync(s.ownedU8[p], s.stageHost + p * planeBytes, planeBytes, cudaMemcpyHostToDevice, c->stream));      // overlaps the packing of the next plane
-            s.d.planeU8[p] = s.ownedU8[p];
-            s.d.plane[p] = s.owned[p];
         }
         CK(cudaEventRecord(s.stageFree, c->stream));
         s.stageBusy = true;
-        s.d.isU8 = 1; s.d.pitchU8 = (int)pitch;
-        s.int32Valid = false;
+        if (!(bad & ~255u)) return use_packed_planes(c, slot);
         // samples outside 0..255 (signed chroma planes): this image goes up as int32 instead.  yk_range_dyn takes such
         // planes; the alpha / gradient / 1-D range stages report YK_ERR_RANGE for them either way.
-        if (bad & ~255u) packed = false;
     }
-    if (!packed) {
-        for (int p = 0; p < nPlanes; p++) {
-            CK(cudaMemcpyAsync(s.owned[p], planes[p], (size_t)w * h * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-            s.d.plane[p] = s.owned[p];
-            s.d.planeU8[p] = nullptr;
-        }
-        s.d.isU8 = 0; s.d.pitchU8 = 0;
-        s.int32Valid = true;
+    for (int p = 0; p < nPlanes; p++) {
+        CK(cudaMemcpyAsync(s.owned[p], planes[p], (size_t)w * h * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+        s.d.plane[p] = s.owned[p];
+        s.d.planeU8[p] = nullptr;
     }
+    s.d.isU8 = 0; s.d.pitchU8 = 0;
+    s.int32Valid = true;
     for (int p = nPlanes; p < 4; p++) { s.d.plane[p] = nullptr; s.d.planeU8[p] = nullptr; }
     s.borrowed = false;
     if ((rc = encode_slot_tmaps(s))) return rc;
@@ -504,6 +518,47 @@ extern "C" int yk_set_image_device(yk_ctx* c, int slot, const int32_t* const* de
     s.borrowed = true;
     if ((rc = encode_slot_tmaps(s))) return rc;
     return yk_reset_state(c, slot);
+}
+
+// Interleaved 8-bit pixels at `src` (device memory, or the context's staging copy) into the slot's packed planes
+static int unpack_interleaved(yk_ctx* c, int slot, const uint8_t* src, size_t rowBytes, int channels) {
+    YkSlotHost& s = c->slots[slot];
+    YkUnpackArgs a;
+    a.src = src; a.rowBytes = rowBytes; a.nPlanes = s.d.nPlanes; a.w = s.d.w; a.h = s.d.h; a.pitch = (s.d.w + 15) / 16 * 16;
+    for (int p = 0; p < 4; p++) a.dst[p] = p < s.d.nPlanes ? s.ownedU8[p] : nullptr;
+    { YkTimed t(c, 5); yk_launch_unpack8(a, channels, c->stream); }
+    c->launches++;
+    CK(cudaGetLastError());
+    return use_packed_planes(c, slot);
+}
+
+static int check_interleaved(yk_ctx* c, int slot, const uint8_t* pixels, size_t rowBytes, int channels, int nPlanes, int w, int h) {
+    if (!slot_ok(c, slot) || !pixels || (channels != 3 && channels != 4) || (nPlanes != 3 && nPlanes != channels)) return YK_ERR_ARG;
+    if (w < 0 || rowBytes < (size_t)w * channels) return YK_ERR_ARG;
+    return configure_slot(c, slot, nPlanes, w, h);
+}
+
+extern "C" int yk_set_image_interleaved(yk_ctx* c, int slot, const uint8_t* pixels, size_t rowBytes, int channels, int nPlanes, int w, int h) {
+    int rc = check_interleaved(c, slot, pixels, rowBytes, channels, nPlanes, w, h);
+    if (rc) return rc;
+    CK(cudaSetDevice(c->device));
+    // one copy of the span from the first pixel to the last pixel's last byte, never past it (a decoder's buffer often ends there)
+    const size_t need = rowBytes * (h - 1) + (size_t)w * channels;
+    if (c->stage8Bytes < need) {
+        if (c->stage8) { CK(cudaStreamSynchronize(c->stream)); cudaFree(c->stage8); }
+        c->stage8 = nullptr; c->stage8Bytes = 0;
+        CK(cudaMalloc((void**)&c->stage8, need));
+        c->stage8Bytes = need;
+    }
+    CK(cudaMemcpyAsync(c->stage8, pixels, need, cudaMemcpyHostToDevice, c->stream));
+    return unpack_interleaved(c, slot, c->stage8, rowBytes, channels);
+}
+
+extern "C" int yk_set_image_interleaved_device(yk_ctx* c, int slot, const uint8_t* devPixels, size_t rowBytes, int channels, int nPlanes, int w, int h) {
+    int rc = check_interleaved(c, slot, devPixels, rowBytes, channels, nPlanes, w, h);
+    if (rc) return rc;
+    CK(cudaSetDevice(c->device));
+    return unpack_interleaved(c, slot, devPixels, rowBytes, channels);
 }
 
 extern "C" int32_t* yk_device_plane(yk_ctx* c, int slot, int p) {

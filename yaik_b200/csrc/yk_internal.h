@@ -152,6 +152,9 @@ int  yk_preload_emit();
 int  yk_preload_aux();      // opt-in shared memory of the persistent kernel; returns a cudaError_t
 void yk_launch_analyze(const YkSlotDev* slotsDev, int slot0, int nSlots, int nRegions, int gridCtas, bool packedU8, const YkRun& run, cudaStream_t st);   // nRegions: of one image (nbx * nby)
 void yk_launch_expand(const YkSlotDev* slotsDev, int slot, int nPlanes, int w, int h, int32_t* const* dst, cudaStream_t st);
+// interleaved 8-bit pixels (channels 3 or 4, rows rowBytes apart) -> nPlanes packed planes of row pitch `pitch` (yk_k_unpack8)
+struct YkUnpackArgs { const uint8_t* src; size_t rowBytes; int nPlanes, w, h, pitch; uint8_t* dst[4]; };
+void yk_launch_unpack8(const YkUnpackArgs& a, int channels, cudaStream_t st);
 void yk_launch_fold_touch(const YkSlotDev* slotsDev, int slot0, int nSlots, int nWords, cudaStream_t st);
 // one-thread kernels on a strip's stream: publish / wait for an epoch number in (peer-mapped) halo memory
 void yk_launch_flag_set(unsigned* a, unsigned* b, unsigned value, cudaStream_t st);

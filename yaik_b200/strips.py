@@ -119,13 +119,16 @@ class LocalTransport:
             merged["alpha"] = merge_alpha(L, [ctx.alpha_kept() for ctx in ctxs], w, h)
         return merged
 
-    def run(self, planes: np.ndarray, n_strips=None, reject=3, r2=True):
+    def run(self, planes: np.ndarray, n_strips=None, reject=3, r2=True, load=None):
+        """load(ctx, y0, h): puts rows [y0, y0 + h) of the image into slot 0 of ctx (default: yk_set_image of those rows of
+        `planes`); e.g. a pointer y0 * rowBytes into one interleaved image, with no copy on the host."""
         c, h, w = planes.shape
         rows = strip_rows(h, n_strips or len(self.ctxs))
         ctxs = self.ctxs[:len(rows)]
+        load = load or (lambda ctx, y0, sh: ctx.set_image(planes[:, y0:y0 + sh], 0))
         halos = []
         for ctx, (y0, sh) in zip(ctxs, rows):
-            ctx.set_image(planes[:, y0:y0 + sh], 0)
+            load(ctx, y0, sh)
             ctx.strip_config(h, y0)
             halos.append(ctx.strip_halo())
         # exchange 1: first pixel row of strip k+1 -> halo of strip k
