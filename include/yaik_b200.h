@@ -225,7 +225,8 @@ int  yk_profile_read(yk_ctx* ctx, double ms[8], long long count[8]);
  * and the per-pass getters return the strip's part: bitmaps are consecutive byte ranges of the image's
  * bitmaps, rgb / range streams concatenate in strip order, TileDone adds up, boxes merge (they are in image
  * coordinates).  The two exchanges are plain device-to-device copies (NVLink P2P through CUDA IPC between
- * the per-GPU processes), never a collective.  Only the fused 7-pass form on a fresh state is provided. */
+ * the per-GPU processes), never a collective.  Only the fused 7-pass form on a fresh state is provided, plus
+ * DynamicTileEncode of R, G, B (yk_strip_range_dyn below); the chroma front-end is not provided for strips. */
 typedef struct yk_strip_halo {
     void*  haloIn;                 /* one device allocation of this strip, written by its neighbours */
     size_t haloBytes;
@@ -240,6 +241,20 @@ typedef struct yk_strip_halo {
 int  yk_strip_config(yk_ctx* ctx, int slot, int imgH, int y0);
 int  yk_strip_halo_ptrs(yk_ctx* ctx, int slot, yk_strip_halo* out);
 int  yk_strip_phase(yk_ctx* ctx, int slot, int phase, int rejectFactor);  /* 0 = accept phase, 1 = emission phase */
+/* DynamicTileEncode (EC.cpp:4365-4503) of the strip's rows, R, G and B in one launch pair, after phase 0 (an 8x8 block
+ * needs only its own samples, its cells' claimed bits and the alpha mask, so it needs no halo).  The strip codes exactly
+ * the blocks of the whole image's LeftRightOrder walk whose top row it holds, with the image's geometry (constraint box,
+ * block sizes).  imageBoundPx: the strip set's merged alpha box for 4 planes (strips.merge_alpha / yk_alpha_assemble),
+ * NULL for 3 planes (the whole image); the alpha mask applies unless that box is the whole image (EC.cpp:1400-1403).
+ * Enqueued only, no synchronisation.  yk_range_dyn(..., dst = NULL) on the strip then returns the strip's part of each
+ * plane's streams: nibbles and defs start at 0 for every strip, and the strips' parts concatenated in strip order are the
+ * image's streams (every part has an even nibble count); `constraint` is the image's box.  yk_range_dyn on a strip returns
+ * YK_ERR_STATE if the strip was not coded in that mode and YK_ERR_UNSUPPORTED for dst != NULL.
+ * YK_ERR_ARG: the box is empty or outside [0, w) x [0, imgH), a box for 3 planes, none for 4, or w / imgH not multiples
+ * of 8 or below 32.  YK_ERR_STATE: not a strip, or phase 0 has not run on this image.
+ * Not provided for strips: the chroma front-end (the reduced planes' min/max rule reads mask rows of other strips,
+ * Plane.cpp:516) and the write-back plane. */
+int  yk_strip_range_dyn(yk_ctx* ctx, int slot, int mode3BitOnly, const int imageBoundPx[4]);
 /* The same protocol without the host in the loop: after yk_strip_config on every strip (and one host barrier, so that
  * every halo is cleared before a neighbour writes into it) each strip is told where its neighbours' halo allocations
  * are mapped in this process (their haloIn, direct or through yk_ipc_open; NULL where there is no neighbour), and
@@ -247,13 +262,20 @@ int  yk_strip_phase(yk_ctx* ctx, int slot, int phase, int rejectFactor);  /* 0 =
  * The exchanges are peer copies followed by a one-thread kernel that publishes an epoch number in the neighbour's halo;
  * a one-thread kernel on the receiving stream waits for it, and a strip does not start the next image before both
  * neighbours have finished the current one.  Images can be enqueued back to back; the planes must stay what
- * yk_set_image / yk_set_image_device made them. */
+ * yk_set_image / yk_set_image_device made them.  yk_strip_set_peers also makes the R1 tables resident (it synchronises
+ * the stream on first use); yk_strip_run never makes the host wait.
+ * yk_strip_run_stages: stages = 0, YK_STAGE_RANGEDYN or YK_STAGE_RANGEDYN3 (any other bit: YK_ERR_ARG) adds
+ * DynamicTileEncode of the strip (as yk_strip_range_dyn with the whole image as box) between exchange 2 and phase 1,
+ * while the touch words travel.  3 planes only: with R1, an RGBA strip returns YK_ERR_UNSUPPORTED before anything is
+ * enqueued (its alpha box is a reduction over all strips, not a neighbour exchange).  yk_strip_run = stages 0. */
 int  yk_strip_set_peers(yk_ctx* ctx, int slot, void* aboveHalo, void* belowHalo);
 int  yk_strip_run(yk_ctx* ctx, int slot, int rejectFactor);
+int  yk_strip_run_stages(yk_ctx* ctx, int slot, int rejectFactor, int stages);
 /* All strips of an image driven by one process (ctxs[k] = strip k, top to bottom, on one or several GPUs): link every
  * strip to its neighbours (peer access is enabled between their devices), enqueue one image on every strip. */
 int  yk_strips_link(yk_ctx* const* ctxs, int n, int slot);
 int  yk_strips_run(yk_ctx* const* ctxs, int n, int slot, int rejectFactor);
+int  yk_strips_run_stages(yk_ctx* const* ctxs, int n, int slot, int rejectFactor, int stages);    /* every strip checked before any is enqueued */
 /* Alpha stage of a strip set (yk_alpha_reject serves whole images): the per-16x16-tile "has a non-zero alpha sample" bytes of
  * one strip ([tilesH][tilesW], row-major) with the box of its kept tiles in image coordinates, and the assembly of
  * MipPrefilter's results (EC.cpp:1287-1403) from the strips' arrays one after the other and the merged box: host code. */

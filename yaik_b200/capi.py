@@ -27,6 +27,7 @@ EXPORTS = [
     "yk_gradient_pass", "yk_range1d", "yk_range_dyn", "yk_chroma_prepare", "yk_chroma_plane", "yk_range_dyn_chroma", "yk_download_state", "yk_fetch_all", "yk_result_bytes", "yk_launch_count",
     "yk_profile", "yk_profile_read",
     "yk_strip_config", "yk_strip_halo_ptrs", "yk_strip_phase", "yk_strip_set_peers", "yk_strip_run", "yk_strips_link", "yk_strips_run", "yk_alpha_kept", "yk_alpha_assemble",
+    "yk_strip_range_dyn", "yk_strip_run_stages", "yk_strips_run_stages",
     "yk_ipc_export", "yk_ipc_open", "yk_ipc_close", "yk_copy_async", "yk_copy_to_host", "yk_copy_from_host",
     "yk_palette_create", "yk_palette_destroy", "yk_palette_reset", "yk_palette_compress",
     "yk_chunk_file_header", "yk_chunk_mipm", "yk_chunk_gtil", "yk_chunk_1dtl", "yk_chunk_plnt", "yk_chunk_end",
@@ -115,6 +116,9 @@ def load_library(path: str | None = None):
     L.yk_strip_run.argtypes = [C.c_void_p, C.c_int, C.c_int]
     L.yk_strips_link.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_int]
     L.yk_strips_run.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_int]
+    L.yk_strip_range_dyn.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int)]
+    L.yk_strip_run_stages.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int]
+    L.yk_strips_run_stages.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_int, C.c_int]
     L.yk_alpha_kept.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
     L.yk_alpha_assemble.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.c_void_p, C.c_int, C.POINTER(C.c_int),
                                     C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
@@ -328,8 +332,15 @@ class Context:
     def strip_set_peers(self, above, below, slot=0):
         self._ck(self.L.yk_strip_set_peers(self.ctx, slot, C.c_void_p(above or 0), C.c_void_p(below or 0)), "yk_strip_set_peers")
 
-    def strip_run(self, slot=0, reject=3):
-        self._ck(self.L.yk_strip_run(self.ctx, slot, reject), "yk_strip_run")
+    def strip_run(self, slot=0, reject=3, stages=0):
+        """One image without the host in the loop; stages = 0, STAGE_RANGEDYN or STAGE_RANGEDYN3 (R1 of an RGB strip)."""
+        self._ck(self.L.yk_strip_run_stages(self.ctx, slot, reject, stages), "yk_strip_run_stages")
+
+    def strip_range_dyn(self, mode3=False, bound=None, slot=0):
+        """DynamicTileEncode of the strip's rows after phase 0 (range_dyn then returns the strip's part).  bound: the strip
+        set's merged alpha box for RGBA (strips.merge_alpha), None for RGB."""
+        box = (C.c_int * 4)(*bound) if bound is not None else None
+        self._ck(self.L.yk_strip_range_dyn(self.ctx, slot, int(mode3), box), "yk_strip_range_dyn")
 
     def alpha_kept(self, slot=0):
         """Per-tile alpha results of one strip (or image): kept bytes [th][tw], box of the kept tiles in image coordinates."""

@@ -83,6 +83,9 @@ struct YkSlotHost {
     size_t haloFlagsOffset = 0;  // five u32 epoch flags written by the neighbours: see yk_strip_run
     void* peerAbove = nullptr; void* peerBelow = nullptr;     // the neighbours' halo allocations as mapped in this process
     unsigned stripEpoch = 0;
+    bool strip = false;          // yk_strip_config placed the current image in a strip set
+    int  r1Strip = 0;            // DynamicTileEncode of the strip's rows present (yk_strip_range_dyn): 1 = six modes, 2 = 3-bit only
+    int  r1StripConstraint[4] = { 0, 0, 0, 0 };     // ... and the image's constraint box it was coded in
 };
 
 struct yk_ctx {
@@ -109,6 +112,9 @@ struct yk_ctx {
     // grown on demand.  One per context is enough: stream order puts every copy into it after the unpack of the previous one.
     // Its base is 256-byte aligned, so 16-byte aligned rows take yk_k_unpack8's vector path whatever the caller's base.
     uint8_t* stage8 = nullptr; size_t stage8Bytes = 0;
+    // set while yk_strip_run_stages enqueues: the steps that would make the host wait for the stream (a pageable
+    // descriptor upload, a header copy-back, the first upload of the R1 tables) fail with YK_ERR_STATE instead
+    bool noHostWait = false;
 };
 
 struct YkTimed {        // records an event pair around one launch when profiling is on
@@ -388,7 +394,7 @@ static int configure_slot(yk_ctx* c, int slot, int nPlanes, int w, int h) {
     s.d.imgH = h; s.d.y0 = 0; s.d.hasAbove = 0; s.d.hasBelow = 0; s.d.touchInTop = nullptr; s.d.touchInBottom = nullptr;
     s.d.latW = w / 4 + 1; s.d.latH = h / 4 + 1;
     for (int p = 0; p < 3; p++) s.d.rowBelow[p] = nullptr;
-    s.haveImage = true; s.dirty = true; s.chromaReady = false;
+    s.haveImage = true; s.dirty = true; s.chromaReady = false; s.strip = false;
     return YK_OK;
 }
 
@@ -397,7 +403,7 @@ static void mark_reset(YkSlotHost& s) {
     if (s.d.alphaReset || s.d.alphaValid) s.dirty = true;
     s.d.alphaReset = 0; s.d.alphaValid = 0;
     s.k1Ran = s.alphaRan = s.alphaFetched = s.prepared = s.r2Valid = s.pendingHarvest = false;
-    s.r1Fused = 0;
+    s.r1Fused = 0; s.r1Strip = 0;
     s.nextPass = 0; s.rangeErr = 0; s.lastRunPasses = 0;
     memset(s.hdr, 0, sizeof s.hdr);
 }
@@ -572,6 +578,7 @@ static int upload_slots(yk_ctx* c, int slot0, int nSlots) {
     for (int i = slot0; i < slot0 + nSlots; i++) {
         YkSlotHost& s = c->slots[i];
         if (s.dirty) {
+            if (c->noHostWait) return YK_ERR_STATE;
             CK(cudaMemcpyAsync(c->slotsDev + i, &s.d, sizeof(YkSlotDev), cudaMemcpyHostToDevice, c->stream));
             s.dirty = false;
         }
@@ -594,6 +601,7 @@ static int check_batch(yk_ctx* c, int slot0, int nSlots) {
 // alpha box if it ran the alpha stage, the R2 totals (the scan always refreshes them).
 static int fetch_hdr(yk_ctx* c, YkSlotHost& s) {
     if (s.pendingHarvest) {
+        if (c->noHostWait) return YK_ERR_STATE;
         int tmp[YK_HD_INTS];
         CK(cudaMemcpyAsync(tmp, s.d.hdr, sizeof tmp, cudaMemcpyDeviceToHost, c->stream));
         CK(cudaStreamSynchronize(c->stream));
@@ -954,6 +962,7 @@ static const YkR1HostTables& r1_host_tables() {
 }
 static int ensure_r1_lut(yk_ctx* c) {
     if (c->lutDev && c->rtabDev && c->r7Dev) return YK_OK;
+    if (c->noHostWait) return YK_ERR_STATE;
     const YkR1HostTables& t = r1_host_tables();
     if (!t.ok) return YK_ERR_STATE;
     CK(cudaMalloc((void**)&c->lutDev, t.lut.size() * sizeof(int)));
@@ -1073,6 +1082,13 @@ extern "C" int yk_range_dyn(yk_ctx* c, int slot, int plane, int mode3BitOnly, ui
     if (!s.haveImage) return YK_ERR_STATE;
     CK(cudaSetDevice(c->device));
     int rc;
+    if (s.strip) {
+        // the strip's part of the image's streams, as the last yk_strip_range_dyn / yk_strip_run_stages coded them
+        if (dst) return YK_ERR_UNSUPPORTED;
+        if (s.r1Strip != (mode3BitOnly ? 2 : 1)) return YK_ERR_STATE;
+        if (constraint) memcpy(constraint, s.r1StripConstraint, sizeof s.r1StripConstraint);
+        return r1_fetch(c, s, plane, nibbles, nibCap, nNibbles, defs, defsCap, nDefs);
+    }
     if (!dst && s.r1Fused == (mode3BitOnly ? 2 : 1)) {
         // coded by yk_analyze already: only the streams come back
         YkR1Walk g;
@@ -1263,6 +1279,7 @@ extern "C" int yk_strip_config(yk_ctx* c, int slot, int imgH, int y0) {
     s.d.touchInBottom = (const uint32_t*)(s.haloIn + 3 * rowBytes + touchBytes);
     s.haloFlagsOffset = 3 * rowBytes + 2 * touchBytes;
     s.stripEpoch = 0; s.peerAbove = nullptr; s.peerBelow = nullptr;
+    s.strip = true; s.r1Strip = 0;
     s.dirty = true;
     return YK_OK;
 }
@@ -1305,6 +1322,61 @@ extern "C" int yk_strip_phase(yk_ctx* c, int slot, int phase, int rejectFactor) 
     return YK_OK;
 }
 
+// ---- DynamicTileEncode of a strip -----------------------------------------------------------------------------------
+// An 8x8 block depends on its own samples, its 4x4 cells' claimed bits (final after phase 0) and the alpha mask, and strips
+// start on multiples of 64: each strip codes the blocks of the image's walk whose top row it holds, with the image's
+// geometry.  The image's constraint box and the mask decision are the only global inputs (imageBoundPx: the strip set's
+// merged alpha box, or the whole image).  Each strip's streams start at 0; concatenated in strip order they are the image's.
+static int r1_strip_args(const YkSlotHost& s, const int imageBoundPx[4]) {
+    const int w = s.d.w, imgH = s.d.imgH;
+    if ((w & 7) || (imgH & 7) || w < 32 || imgH < 32) return YK_ERR_ARG;      // the reference's own domain (SURVEY.md hazard 11)
+    if ((s.d.nPlanes == 4) != (imageBoundPx != nullptr)) return YK_ERR_ARG;   // RGBA: the merged alpha box; RGB: the whole image
+    if (imageBoundPx) {
+        const int L = imageBoundPx[0], T = imageBoundPx[1], R = imageBoundPx[2], B = imageBoundPx[3];
+        if (L < 0 || T < 0 || R > w || B > imgH || L >= R || T >= B) return YK_ERR_ARG;
+    }
+    return YK_OK;
+}
+
+// enqueues the three-plane pair (yk_k_r1_offsets + yk_k_r1_encode3) over the strip's window; no synchronisation
+static int enqueue_r1_strip(yk_ctx* c, int slot, int mode3BitOnly, const int imageBoundPx[4]) {
+    YkSlotHost& s = c->slots[slot];
+    const int w = s.d.w, imgH = s.d.imgH;
+    const int full[4] = { 0, 0, w, imgH };
+    const int* box = imageBoundPx ? imageBoundPx : full;
+    // mipmapMask holds the alpha stage's rejection unless the box is the whole image (EC.cpp:1400-1403)
+    const int maskValid = s.d.nPlanes == 4, maskReset = maskValid && yk_box_is_image(box, w, imgH);
+    if (s.d.alphaValid != maskValid || s.d.alphaReset != maskReset) { s.d.alphaValid = maskValid; s.d.alphaReset = maskReset; s.dirty = true; }
+    int rc;
+    if ((rc = upload_slots(c, slot, 1))) return rc;
+    YkR1Launch L;
+    memset(&L, 0, sizeof L);
+    L.nJobs = 3; L.mode3 = mode3BitOnly ? 1 : 0;
+    L.pw = w; L.ph = imgH;
+    const YkR1Walk g = yk_r1_walk(box, imgH, 0, 0);
+    L.walk = yk_r1_window(g, s.d.y0, s.d.h);
+    for (int p = 0; p < 3; p++) {
+        YkR1Args& a = L.job[p];
+        a.src = s.d.plane[p]; a.srcU8 = s.d.isU8 ? s.d.planeU8[p] : nullptr; a.pitchU8 = s.d.pitchU8; a.out = p;
+    }
+    s.r1Strip = 0;                                               // the streams are about to be replaced
+    if ((rc = launch_r1(c, slot, L))) return rc;
+    s.r1Strip = mode3BitOnly ? 2 : 1;
+    s.r1StripConstraint[0] = g.cx; s.r1StripConstraint[1] = g.cy; s.r1StripConstraint[2] = g.cw; s.r1StripConstraint[3] = g.ch;
+    return YK_OK;
+}
+
+extern "C" int yk_strip_range_dyn(yk_ctx* c, int slot, int mode3BitOnly, const int imageBoundPx[4]) {
+    if (!slot_ok(c, slot)) return YK_ERR_ARG;
+    YkSlotHost& s = c->slots[slot];
+    if (!s.haveImage || !s.strip) return YK_ERR_STATE;
+    int rc;
+    if ((rc = r1_strip_args(s, imageBoundPx))) return rc;
+    if (s.cellsClean) return YK_ERR_STATE;                         // phase 0 has not run on this image
+    CK(cudaSetDevice(c->device));
+    return enqueue_r1_strip(c, slot, mode3BitOnly, imageBoundPx);
+}
+
 // ---- strips without the host in the loop ----------------------------------------------------------------------------
 // Every strip enqueues the whole image on its own stream: the two exchanges are device-to-device copies into the
 // neighbours' halo allocations (peer-mapped: NVLink P2P), each followed by a one-thread kernel that publishes an epoch
@@ -1317,26 +1389,45 @@ extern "C" int yk_strip_set_peers(yk_ctx* c, int slot, void* aboveHalo, void* be
     YkSlotHost& s = c->slots[slot];
     if (!s.haveImage || !s.haloIn) return YK_ERR_STATE;
     if ((s.d.hasAbove && !aboveHalo) || (s.d.hasBelow && !belowHalo)) return YK_ERR_ARG;
+    // the R1 tables go up now, while waiting for this stream is harmless: yk_strip_run_stages must not wait
+    CK(cudaSetDevice(c->device));
+    const int rc = ensure_r1_lut(c);
+    if (rc) return rc;
     s.peerAbove = s.d.hasAbove ? aboveHalo : nullptr; s.peerBelow = s.d.hasBelow ? belowHalo : nullptr;
     return YK_OK;
 }
 
-extern "C" int yk_strip_run(yk_ctx* c, int slot, int rejectFactor) {
+static int strip_run_check(yk_ctx* c, int slot, int rejectFactor, int stages) {
     if (!slot_ok(c, slot) || rejectFactor < 0 || rejectFactor > 64) return YK_ERR_ARG;
+    const int r1 = stages & (YK_STAGE_RANGEDYN | YK_STAGE_RANGEDYN3);
+    if ((stages & ~r1) || r1 == (YK_STAGE_RANGEDYN | YK_STAGE_RANGEDYN3)) return YK_ERR_ARG;
     YkSlotHost& s = c->slots[slot];
     if (!s.haveImage || !s.haloIn) return YK_ERR_STATE;
     if ((s.d.hasAbove && !s.peerAbove) || (s.d.hasBelow && !s.peerBelow)) return YK_ERR_STATE;
-#ifdef YK_EMULATE
-    return YK_ERR_UNSUPPORTED;      // the emulated launches run to completion one after the other: a waiting kernel would never see its flag
-#endif
+    // RGBA: the alpha box is a reduction over every strip, not a neighbour exchange
+    if (r1 && s.d.nPlanes == 4) return YK_ERR_UNSUPPORTED;
+    if (r1) return r1_strip_args(s, nullptr);
+    return YK_OK;
+}
+
+struct YkNoHostWait {       // see yk_ctx::noHostWait
+    yk_ctx* c;
+    explicit YkNoHostWait(yk_ctx* c_) : c(c_) { c->noHostWait = true; }
+    ~YkNoHostWait() { c->noHostWait = false; }
+};
+
+static int strip_run_enqueue(yk_ctx* c, int slot, int rejectFactor, int stages) {
+    YkSlotHost& s = c->slots[slot];
     CK(cudaSetDevice(c->device));
     // Nothing below may make the host wait for this stream: it is about to hold kernels that wait for the neighbours,
     // whose work the same host thread may still have to enqueue.  So the slot descriptor goes up now (a copy from
-    // pageable memory drains the stream first), and the previous image's header is not fetched (its counters are lost
-    // unless they were read before the next yk_strip_run).
+    // pageable memory drains the stream first), with the mask flags yk_reset_state below clears, and the previous
+    // image's header is not fetched (its counters are lost unless they were read before the next run).
+    if (s.d.alphaValid || s.d.alphaReset) { s.d.alphaValid = 0; s.d.alphaReset = 0; s.dirty = true; }
     int rc = upload_slots(c, slot, 1);
     if (rc) return rc;
     s.pendingHarvest = false;
+    YkNoHostWait guard(c);
     const unsigned e = ++s.stripEpoch;
     const size_t es = s.d.isU8 ? 1 : sizeof(int32_t), rowBytes = ((size_t)s.d.w * es + 15) / 16 * 16;
     const size_t touchBytes = (size_t)s.d.latW * sizeof(uint32_t);
@@ -1361,12 +1452,24 @@ extern "C" int yk_strip_run(yk_ctx* c, int slot, int rejectFactor) {
     if (above) CK(cudaMemcpyAsync((uint8_t*)s.peerAbove + offBottom, s.d.touchMap, touchBytes, cudaMemcpyDefault, c->stream));
     if (below) CK(cudaMemcpyAsync((uint8_t*)s.peerBelow + offTop, s.d.touchMap + (size_t)(s.d.latH - 1) * s.d.latW, touchBytes, cudaMemcpyDefault, c->stream));
     if (above || below) { yk_launch_flag_set(above ? above + 2 : nullptr, below ? below + 1 : nullptr, e, c->stream); c->launches++; }
+    // R1 needs nothing from the neighbours: it runs while their touch words travel
+    if ((stages & (YK_STAGE_RANGEDYN | YK_STAGE_RANGEDYN3)) && (rc = enqueue_r1_strip(c, slot, (stages & YK_STAGE_RANGEDYN3) != 0, nullptr))) return rc;
     if (above || below) { yk_launch_flag_wait(above ? mine + 1 : nullptr, below ? mine + 2 : nullptr, e, c->stream); c->launches++; }
     if ((rc = yk_strip_phase(c, slot, 1, rejectFactor))) return rc;
     if (above || below) { yk_launch_flag_set(above ? above + 4 : nullptr, below ? below + 3 : nullptr, e, c->stream); c->launches++; }
     CK(cudaGetLastError());
     return YK_OK;
 }
+
+extern "C" int yk_strip_run_stages(yk_ctx* c, int slot, int rejectFactor, int stages) {
+    const int rc = strip_run_check(c, slot, rejectFactor, stages);
+    if (rc) return rc;
+#ifdef YK_EMULATE
+    return YK_ERR_UNSUPPORTED;      // the emulated launches run to completion one after the other: a waiting kernel would never see its flag
+#endif
+    return strip_run_enqueue(c, slot, rejectFactor, stages);
+}
+extern "C" int yk_strip_run(yk_ctx* c, int slot, int rejectFactor) { return yk_strip_run_stages(c, slot, rejectFactor, 0); }
 
 // all strips of an image driven by this process (one context per strip, on one or several GPUs): link every strip to its
 // neighbours' halo allocations directly, then enqueue an image on every strip
@@ -1391,11 +1494,13 @@ extern "C" int yk_strips_link(yk_ctx* const* ctxs, int n, int slot) {
     }
     return YK_OK;
 }
-extern "C" int yk_strips_run(yk_ctx* const* ctxs, int n, int slot, int rejectFactor) {
+extern "C" int yk_strips_run_stages(yk_ctx* const* ctxs, int n, int slot, int rejectFactor, int stages) {
     if (!ctxs || n < 1) return YK_ERR_ARG;
-    for (int k = 0; k < n; k++) { const int rc = yk_strip_run(ctxs[k], slot, rejectFactor); if (rc) return rc; }
+    for (int k = 0; k < n; k++) { const int rc = strip_run_check(ctxs[k], slot, rejectFactor, stages); if (rc) return rc; }     // nothing enqueued on an error
+    for (int k = 0; k < n; k++) { const int rc = yk_strip_run_stages(ctxs[k], slot, rejectFactor, stages); if (rc) return rc; }
     return YK_OK;
 }
+extern "C" int yk_strips_run(yk_ctx* const* ctxs, int n, int slot, int rejectFactor) { return yk_strips_run_stages(ctxs, n, slot, rejectFactor, 0); }
 
 // ---- alpha stage of a strip set: the per-tile results of one strip, and their assembly (host code) ------------------
 extern "C" int yk_alpha_kept(yk_ctx* c, int slot, uint8_t* kept, int keptCap, int* tilesW, int* tilesH, int boundPx[4], int* keptTiles) {

@@ -129,7 +129,8 @@ static __host__ __device__ inline bool yk_box_is_image(const int box[4], int w, 
 // The walk of LeftRightOrder (framework.h:228-256) over the 8-aligned bound box (EC.cpp:4386-4401), halved on the
 // reduced axes of a plane of ph rows: rows of nbw = ceil(cw / 8) blocks while y < cy + ch, then one more block at the
 // start of the next row when that row still lies inside the plane (HasNextBlock tests `y < h` after the wrap).
-struct YkR1Walk { int cx, cy, cw, ch, nbw, nBlocks; };
+// A launch codes blocks b0 .. b0 + nBlocks - 1 of the walk (all of them, or the window of a tile-row strip).
+struct YkR1Walk { int cx, cy, cw, ch, nbw, nBlocks, b0; };
 static __host__ __device__ inline YkR1Walk yk_r1_walk(const int box[4], int ph, int shX, int shY) {
     YkR1Walk g;
     g.cx = (box[0] >> 3) << 3; g.cy = (box[1] >> 3) << 3;                              // EC.cpp:4386-4391
@@ -139,6 +140,18 @@ static __host__ __device__ inline YkR1Walk yk_r1_walk(const int box[4], int ph, 
     const int rows = (g.ch + 7) >> 3;
     g.nBlocks = g.nbw * rows;
     if (g.nBlocks > 0 && g.cy + 8 * rows < ph) g.nBlocks += 1;
+    g.b0 = 0;
+    return g;
+}
+// The window of a whole-image walk g that a tile-row strip of rows [y0, y0 + h) codes: the blocks whose top row (image
+// coordinates) lies in the strip, the extra block after the last row included.  Rows are whole walk rows, so the
+// strips' windows cut the walk into consecutive pieces.
+static __host__ __device__ inline YkR1Walk yk_r1_window(YkR1Walk g, int y0, int h) {
+    const int total = g.nBlocks;
+    const int r0 = y0 <= g.cy ? 0 : (y0 - g.cy + 7) >> 3, r1 = y0 + h <= g.cy ? 0 : (y0 + h - g.cy + 7) >> 3;     // first walk row at or below y0, y0 + h
+    const long long first = (long long)r0 * g.nbw, end = (long long)r1 * g.nbw;
+    g.b0 = (int)(first < total ? first : total);
+    g.nBlocks = (int)(end < total ? end : total) - g.b0;
     return g;
 }
 

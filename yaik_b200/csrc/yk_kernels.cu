@@ -228,14 +228,15 @@ static __device__ __forceinline__ unsigned yk_r1_cells(const YkSlotDev& S, bool 
     return (~(((r0 >> (cx & 15)) & 3u) | (((r1 >> (cx & 15)) & 3u) << 2))) & 15u;
 }
 
-// Block i of the walk is (cx + 8*(i % nbw), cy + 8*(i / nbw)).  Block sizes: the reference compares with the
+// Block b0 + i of the walk is (cx + 8*(j % nbw), cy + 8*(j / nbw)), j = b0 + i, in image coordinates.  Block sizes: the reference compares with the
 // constraint's width / height, not its right / bottom edge, and falls back to x % 8 (framework.h:251-252) - 0 for the
 // full-resolution planes (x + 8 > cw empties the block), possibly 4 for a reduced chroma plane whose box starts on an
 // odd multiple of 4.
 struct YkR1Block { int x, y, rw, rh; };
 static __device__ __forceinline__ YkR1Block yk_r1_block(const YkR1Walk& G, int i) {
     YkR1Block b;
-    b.x = G.cx + 8 * (i % G.nbw); b.y = G.cy + 8 * (i / G.nbw);
+    const int j = G.b0 + i;
+    b.x = G.cx + 8 * (j % G.nbw); b.y = G.cy + 8 * (j / G.nbw);
     b.rw = (b.x + 8 > G.cw) ? (b.x & 7) : 8;
     b.rh = (b.y + 8 > G.ch) ? (b.y & 7) : 8;
     return b;
@@ -304,6 +305,9 @@ yk_k_r1_offsets(const YkSlotDev* __restrict__ slots, int slot, const YkR1Launch 
     if (i < G.nBlocks) {
         b = yk_r1_block(G, i);
         if (!reduced) {
+            // the geometry is the image's; the masks, and the samples the encode kernels read from the list entry, are
+            // the strip's rows (y0 == 0 for a whole image)
+            b.y -= S.y0;
             if (b.rw == 8 && b.rh == 8 && b.x + 8 <= S.w && b.y + 8 <= S.h) {
                 const unsigned cells = yk_r1_cells(S, maskActive, b.x, b.y);
                 pairs = ((cells & 1u) ? 0x00003333u : 0u) | ((cells & 2u) ? 0x0000CCCCu : 0u) | ((cells & 4u) ? 0x33330000u : 0u) | ((cells & 8u) ? 0xCCCC0000u : 0u);

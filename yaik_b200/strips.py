@@ -8,6 +8,10 @@ So an image is cut into strips of whole 64-row swizzle blocks, each strip is an 
     exchange 1   first pixel row of strip k+1  ->  halo of strip k          (before ``yk_strip_phase 0``)
     exchange 2   boundary touch words, both directions                       (between phase 0 and phase 1)
 
+DynamicTileEncode (R1) of R, G, B needs no halo: after phase 0 each strip codes the blocks of the image's walk whose top
+row it holds (``yk_strip_range_dyn``, with the strip set's merged alpha box for RGBA), and its streams are its slice of
+the image's.
+
 Host logic here: the partition, the order of the steps, and the merge of the per-strip results into the image's streams
 (bitmaps are consecutive byte ranges, rgb / range streams concatenate in strip order, TileDone adds, boxes merge).
 Transports: ``LocalTransport`` (all strips driven by this process: direct peer copies), ``DistTransport`` (one strip per
@@ -39,15 +43,26 @@ def strip_rows(img_h: int, n: int):
     return out
 
 
-def collect_results(ctx: "capi.Context", slot=0, r2=True):
-    """Per-strip results through the ordinary getters (after phase 1)."""
+def collect_results(ctx: "capi.Context", slot=0, r2=True, r1=0):
+    """Per-strip results through the ordinary getters (after phase 1).  r1 = STAGE_RANGEDYN / STAGE_RANGEDYN3: also the
+    strip's DynamicTileEncode streams of R, G, B in that mode (res["r1"], one Context.range_dyn dict per plane)."""
     res = {"passes": [], "r2": []}
     for sx, sy in capi.PASS_ORDER:
         res["passes"].append(ctx.gradient_pass(sx, sy, slot))
     if r2:
         for p in range(3):
             res["r2"].append(ctx.range1d(p, slot))
+    if r1:
+        res["r1"] = [ctx.range_dyn(p, mode3=r1 == capi.STAGE_RANGEDYN3, slot=slot) for p in range(3)]
     return res
+
+
+def merged_box(parts):
+    """The image's alpha box from the strips' (bound, kept-tile count) pairs: None when no strip kept a tile."""
+    boxes = [b for b, n in parts if n > 0]
+    if not boxes:
+        return None
+    return [min(b[0] for b in boxes), min(b[1] for b in boxes), max(b[2] for b in boxes), max(b[3] for b in boxes)]
 
 
 def merge_alpha(lib, parts, w, h):
@@ -55,10 +70,9 @@ def merge_alpha(lib, parts, w, h):
     the arrays stack (a strip is a whole number of 16-row tiles, except the last), the boxes merge, the bitmap / remaining
     pixels / chunk box come from yk_alpha_assemble (EC.cpp:1287-1403)."""
     kept = np.ascontiguousarray(np.concatenate([p["kept"] for p in parts], axis=0))
-    boxes = [p["bound"] for p in parts if p["count"] > 0]
-    if not boxes:
+    bound = merged_box([(p["bound"], p["count"]) for p in parts])
+    if bound is None:
         return None                                  # fully transparent: outside the reference's domain
-    bound = [min(b[0] for b in boxes), min(b[1] for b in boxes), max(b[2] for b in boxes), max(b[3] for b in boxes)]
     th, tw = kept.shape
     bm = np.zeros(tw * th // 8 + 8, np.uint8)
     nb, rem, wrote = C.c_int(), C.c_int(), C.c_int()
@@ -84,6 +98,15 @@ def merge_results(parts):
         for pl in range(3):
             out["r2"].append(dict(idx=np.concatenate([p["r2"][pl]["idx"] for p in parts]),
                                   type=np.concatenate([p["r2"][pl]["type"] for p in parts])))
+    if parts and parts[0].get("r1"):
+        out["r1"] = []
+        for pl in range(3):
+            rs = [p["r1"][pl] for p in parts]
+            # a strip codes whole 4x4 cells: its nibbles fill whole bytes, so the strips' bytes concatenate unshifted
+            assert all(r["n_nibbles"] % 2 == 0 for r in rs), [r["n_nibbles"] for r in rs]
+            assert all(r["constraint"] == rs[0]["constraint"] for r in rs), [r["constraint"] for r in rs]
+            out["r1"].append(dict(nibbles=np.concatenate([r["nibbles"] for r in rs]), n_nibbles=int(sum(r["n_nibbles"] for r in rs)),
+                                  defs=np.concatenate([r["defs"] for r in rs]), dst=None, constraint=list(rs[0]["constraint"])))
     return out
 
 
@@ -93,10 +116,11 @@ class LocalTransport:
     def __init__(self, ctxs):
         self.ctxs = ctxs
 
-    def run_device_flags(self, planes: np.ndarray, n_strips=None, reject=3, r2=True, images=1):
-        """The form without the host in the loop (yk_strips_link / yk_strips_run): every strip enqueues the whole image on
-        its stream, the exchanges are ordered by epoch flags in the halos.  `images` > 1 runs the image that many times
-        back to back (the last run's results are collected)."""
+    def run_device_flags(self, planes: np.ndarray, n_strips=None, reject=3, r2=True, images=1, r1=0):
+        """The form without the host in the loop (yk_strips_link / yk_strips_run_stages): every strip enqueues the whole
+        image on its stream, the exchanges are ordered by epoch flags in the halos.  `images` > 1 runs the image that many
+        times back to back (the last run's results are collected).  r1 = STAGE_RANGEDYN / STAGE_RANGEDYN3: every image
+        also codes R1 (RGB only)."""
         c, h, w = planes.shape
         rows = strip_rows(h, n_strips or len(self.ctxs))
         ctxs = self.ctxs[:len(rows)]
@@ -109,19 +133,20 @@ class LocalTransport:
         if rc:
             raise capi.YaikError(rc, "yk_strips_link")
         for _ in range(images):
-            rc = L.yk_strips_run(arr, len(ctxs), 0, reject)
+            rc = L.yk_strips_run_stages(arr, len(ctxs), 0, reject, r1)
             if rc:
-                raise capi.YaikError(rc, "yk_strips_run")
+                raise capi.YaikError(rc, "yk_strips_run_stages")
         for ctx in ctxs:
             ctx.sync()
-        merged = merge_results([collect_results(ctx, r2=r2) for ctx in ctxs])
+        merged = merge_results([collect_results(ctx, r2=r2, r1=r1) for ctx in ctxs])
         if c == 4:
             merged["alpha"] = merge_alpha(L, [ctx.alpha_kept() for ctx in ctxs], w, h)
         return merged
 
-    def run(self, planes: np.ndarray, n_strips=None, reject=3, r2=True, load=None):
+    def run(self, planes: np.ndarray, n_strips=None, reject=3, r2=True, load=None, r1=0):
         """load(ctx, y0, h): puts rows [y0, y0 + h) of the image into slot 0 of ctx (default: yk_set_image of those rows of
-        `planes`); e.g. a pointer y0 * rowBytes into one interleaved image, with no copy on the host."""
+        `planes`); e.g. a pointer y0 * rowBytes into one interleaved image, with no copy on the host.
+        r1 = STAGE_RANGEDYN / STAGE_RANGEDYN3: DynamicTileEncode of R, G, B after phase 0 (merged["r1"])."""
         c, h, w = planes.shape
         rows = strip_rows(h, n_strips or len(self.ctxs))
         ctxs = self.ctxs[:len(rows)]
@@ -142,6 +167,12 @@ class LocalTransport:
             ctx.strip_phase(0, reject=reject)
         for ctx in ctxs:
             ctx.sync()
+        alpha = None
+        if r1:
+            if c == 4:          # the image's alpha box: a reduction over every strip
+                alpha = merge_alpha(ctxs[0].L, [ctx.alpha_kept() for ctx in ctxs], w, h)
+            for ctx in ctxs:
+                ctx.strip_range_dyn(mode3=r1 == capi.STAGE_RANGEDYN3, bound=alpha["bound"] if alpha else None)
         # exchange 2: boundary touch words, both directions
         for k in range(len(rows) - 1):
             up, lo = halos[k], halos[k + 1]
@@ -151,9 +182,9 @@ class LocalTransport:
             ctx.sync()
         for ctx in ctxs:
             ctx.strip_phase(1, reject=reject)
-        merged = merge_results([collect_results(ctx, r2=r2) for ctx in ctxs])
+        merged = merge_results([collect_results(ctx, r2=r2, r1=r1) for ctx in ctxs])
         if c == 4:
-            merged["alpha"] = merge_alpha(ctxs[0].L, [ctx.alpha_kept() for ctx in ctxs], w, h)
+            merged["alpha"] = alpha or merge_alpha(ctxs[0].L, [ctx.alpha_kept() for ctx in ctxs], w, h)
         return merged
 
 
@@ -180,9 +211,10 @@ class DistTransport:
             r.wait()
         return None if got is None else got.numpy()
 
-    def run(self, my_planes, img_h, rows, reject=3, r2=True):
+    def run(self, my_planes, img_h, rows, reject=3, r2=True, r1=0):
         """rows = strip_rows(img_h, world); my_planes = this rank's rows (or None if the rank has no strip).
-        Returns the merged result on rank 0, None elsewhere."""
+        r1 = STAGE_RANGEDYN / STAGE_RANGEDYN3: DynamicTileEncode of R, G, B after phase 0, in the box gathered from every
+        strip's alpha results (RGBA).  Returns the merged result on rank 0, None elsewhere."""
         dist, ctx, rank = self.dist, self.ctx, self.rank
         n = len(rows)
         active = rank < n
@@ -220,6 +252,17 @@ class DistTransport:
         if active:
             ctx.strip_phase(0, reject=reject)
             ctx.sync()
+        if r1:
+            # the image's alpha box is a reduction over every strip: gathered on the control plane, like the IPC handles
+            mine = None
+            if active and my_planes.shape[0] == 4:
+                a = ctx.alpha_kept()
+                mine = (a["bound"], a["count"])
+            boxes = [None] * self.world
+            dist.all_gather_object(boxes, mine)
+            rgba = any(b is not None for b in boxes)
+            if active:
+                ctx.strip_range_dyn(mode3=r1 == capi.STAGE_RANGEDYN3, bound=merged_box([b for b in boxes if b is not None]) if rgba else None)
         # ---- exchange 2: boundary touch words, both directions
         if self.mode == "ipc":
             if above is not None:
@@ -241,7 +284,7 @@ class DistTransport:
         part = None
         if active:
             ctx.strip_phase(1, reject=reject)
-            part = collect_results(ctx, r2=r2)
+            part = collect_results(ctx, r2=r2, r1=r1)
         for r, ptr in peers.items():
             ctx.ipc_close(ptr)
         parts = [None] * self.world
