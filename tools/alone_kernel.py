@@ -1,5 +1,5 @@
 """Developer tool: yk_k_analyze / yk_k_emit / yk_k_owner timed alone (yk_profile: event pair around each launch) for the
-library named by YK_LIB on the bench texture; no result check (usable with measurement-only builds)."""
+library named by YK_LIB on the bench texture; no result check."""
 import sys, os, ctypes as C
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)

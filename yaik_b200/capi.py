@@ -66,7 +66,7 @@ def bitmap_bytes(w, h, shx, shy):
 
 
 def load_library(path: str | None = None):
-    path = path or os.environ.get("YK_LIB") or LIB_PATH      # YK_LIB: developer override for A/B builds of the same sources
+    path = path or os.environ.get("YK_LIB") or LIB_PATH      # YK_LIB: another build of the same sources (e.g. the AddressSanitizer build of tests/emu)
     if not os.path.exists(path):
         raise ImportError(f"{path} is missing: build it with `python -m yaik_b200.build` (nvcc, sm_100a). "
                           "yaik_b200 has no CPU fallback.")

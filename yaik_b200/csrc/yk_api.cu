@@ -3,9 +3,7 @@
 // There is no CPU path here: every compute entry point needs a CUDA device.
 #include "../../include/yaik_b200.h"
 #include "yk_internal.h"
-#ifndef YK_ENDGAME_UNITS
 #define YK_ENDGAME_UNITS 6      // units per CTA at the end of a full-GPU launch that are taken on demand (yk_analyze.cu, producer)
-#endif
 
 #include <limits.h>
 #include <stdio.h>
@@ -160,8 +158,8 @@ extern "C" void* yk_host_alloc(size_t bytes) {
 }
 extern "C" void yk_host_free(void* p) { if (p) cudaFreeHost(p); }
 
-// look-back words of yk_k_r1_offsets: one per unit of YK_R1_UNIT blocks (yk_kernels.cu; sized for units down to 8) of the (8-aligned, possibly one block larger) bound box, + ticket
-static size_t r1_status_words(int W, int H) { return ((size_t)(W / 8 + 1) * (H / 8 + 1) + 7) / 8 + 2; }
+// look-back words of yk_k_r1_offsets: one per unit of YK_R1_UNIT blocks of the (8-aligned, possibly one block larger) bound box, + ticket
+static size_t r1_status_words(int W, int H) { return ((size_t)(W / 8 + 1) * (H / 8 + 1) + YK_R1_UNIT - 1) / YK_R1_UNIT + 2; }
 
 template <class T> static int dev_alloc(YkSlotHost& s, T** out, size_t count) {
     void* p = nullptr;
@@ -241,7 +239,6 @@ static int create_fill(yk_ctx* c) {
     // CTAs of the persistent analysis kernel (default: one per SM).  Leaving a few SMs free lets the small ownership /
     // emission kernels of another stream run beside it when textures are pipelined over several contexts.
     c->analysisCtas = c->numSMs;
-    { const char* e = getenv("YK_ANALYZE_CTAS"); if (e && atoi(e) > 0 && atoi(e) < c->numSMs) c->analysisCtas = atoi(e); }
     CK(cudaMalloc((void**)&c->slotsDev, sizeof(YkSlotDev) * maxSlots));
     const size_t W = maxW, H = maxH;
     const size_t nbx = (W + 63) / 64, latW = W / 4 + 1, latH = H / 4 + 1;

@@ -25,9 +25,7 @@
 // boundary is touched by tiles of both strips.  Each strip ORs in the words its neighbour computed (touchInTop /
 // touchInBottom); a tile of the upper strip always precedes a tile of the lower strip in a pass's stream, and only the
 // strip that holds the owner tile marks it.
-#ifndef YK_OWNER_THREADS
 #define YK_OWNER_THREADS 256
-#endif
 // The pass ids of a launch in run order, 4 bits each.  A kernel that indexed run.passId with a position known only at run
 // time would copy the whole YkRun to local memory first.
 static __device__ __forceinline__ unsigned yk_pass_ids(const YkRun& run) {

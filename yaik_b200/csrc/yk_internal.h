@@ -38,6 +38,8 @@ enum {
 // neighbouring 64x64 regions plus its right / bottom corner samples: the TMA unit's cost is per box row, so rows are
 // made long), 128 x 16 for alpha; out-of-image samples arrive as zeros and are never used unclamped.
 struct alignas(64) YkTmap { unsigned long long opaque[16]; };
+// YK_EMIT_THREADS, YK_SUPER and YK_EMIT_LIST (yk_emit.cu) can be set with -D: the emulated tests build with small
+// values of them, so that small images span many groups, super-groups and copy rounds.
 #ifndef YK_EMIT_THREADS
 #define YK_EMIT_THREADS 512    // threads of a yk_k_emit CTA == nibble words / range tiles per group (host and device agree on it)
 #endif
@@ -87,7 +89,7 @@ struct alignas(128) YkSlotDev {
     uint8_t*  r2Idx[3];         // the streams in the reference's order (gathered by yk_k_emit)
     uint8_t*  r2Type[3];
     // ---- range stage R1 (DynamicTileEncode)
-    unsigned long long* r1Status;   // look-back words of yk_k_r1_offsets' units (256 blocks of the walk each) + the unit ticket; zeroed per call
+    unsigned long long* r1Status;   // look-back words of yk_k_r1_offsets' units (YK_R1_UNIT = 512 blocks of the walk each) + the unit ticket; zeroed per call
     void*     r1List;           // the blocks that hold valid pixels, in walk order (16 bytes each, see yk_k_r1_offsets)
     uint32_t* r1Nib[3];         // nibble stream (two nibbles per byte, written pairwise)
     uint16_t* r1Defs[3];
@@ -125,6 +127,7 @@ static __host__ __device__ inline bool yk_box_is_image(const int box[4], int w, 
 #define YK_R1_LUT_INTS 144          // six LUTs (16,16,16,8,8,8 entries) and their decision thresholds
 #define YK_R1_RTAB_VALUES 384       // sample values of the per-value table: -128..255, shifted by 128 when the minimum is negative
 #define YK_R1_RTAB_R7 128           // range7 values the per-value table covers: every entry of those LUTs is a byte
+#define YK_R1_UNIT 512              // blocks of the walk per yk_k_r1_offsets CTA (one look-back word each)
 
 // The walk of LeftRightOrder (framework.h:228-256) over the 8-aligned bound box (EC.cpp:4386-4401), halved on the
 // reduced axes of a plane of ph rows: rows of nbw = ceil(cw / 8) blocks while y < cy + ch, then one more block at the

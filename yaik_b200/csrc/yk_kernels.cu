@@ -199,12 +199,7 @@ static __device__ int yk_block_exclusive(int v, int* sWarp, int& total) {
 // rtab: [64][128 range7 < 128][6 modes][384] u16 = code << 8 | LUT entry that search picks, for every value 0..383 (the
 // domain of the reference's tables: samples -128..255, shifted by 128 when the block's minimum is negative), built on
 // the host from the same thresholds: the per-pixel, per-mode work of the mode search is one 16-bit load.
-#ifndef YK_R1_UNIT
-#define YK_R1_UNIT 512
-#endif
-#ifndef YK_R1_THREADS
-#define YK_R1_THREADS 128
-#endif
+#define YK_R1_THREADS 128           // CTA size of the encode kernels
 
 // Validity of one full-resolution pixel as DynamicTileEncode sees it: mipmapMask != 0 (kept by the alpha stage) and
 // smoothMap == 0 (its 4x4 cell not claimed by a gradient tile).
@@ -514,12 +509,8 @@ static __device__ __forceinline__ void yk_r1_output(const YkSlotDev& S, const Yk
 }
 
 // One plane (nJobs == 1): a warp takes a listed block and codes it.
-#ifndef YK_R1_MINB
-#define YK_R1_MINB 9
-#endif
-#ifndef YK_R1_CAP
-#define YK_R1_CAP 12
-#endif
+#define YK_R1_MINB 9                // resident CTAs per SM the register budget is set for
+#define YK_R1_CAP 12                // CTAs per SM at most in a launch
 __global__ void __launch_bounds__(YK_R1_THREADS, YK_R1_MINB)
 yk_k_r1_encode(const YkSlotDev* __restrict__ slots, int slot, const YkR1Launch LP, const int* __restrict__ lut, const unsigned short* __restrict__ rtab, const short* __restrict__ r7tab) {
     __shared__ __align__(16) float sTerm[YK_R1_THREADS / 32][6][64];
@@ -584,12 +575,8 @@ yk_k_r1_encode(const YkSlotDev* __restrict__ slots, int slot, const YkR1Launch L
 // block and codes its three planes in one go.  What a block costs besides its per-pixel work is shared by the planes
 // (list entry, geometry, validity ballots), and the ordered error sums - 64 dependent float adds that one lane per mode
 // has to do whatever the other lanes are up to - run for the 18 (plane, mode) pairs side by side in 18 lanes.
-#ifndef YK_R1_MINB3
 #define YK_R1_MINB3 8
-#endif
-#ifndef YK_R1_CAP3
 #define YK_R1_CAP3 8
-#endif
 __global__ void __launch_bounds__(YK_R1_THREADS, YK_R1_MINB3)
 yk_k_r1_encode3(const YkSlotDev* __restrict__ slots, int slot, const YkR1Launch LP, const int* __restrict__ lut, const unsigned short* __restrict__ rtab, const short* __restrict__ r7tab) {
     __shared__ __align__(16) float sTerm[YK_R1_THREADS / 32][3][6][64];
