@@ -41,9 +41,27 @@ static int pass_id(int shX, int shY) {
     return -1;
 }
 
+// bytes of pass p's accept bitmap (pFillBitMap: `bits` bits per swizzle block) for a w x h image; also the number of
+// nibble words its emission fills (4 bits for each of 8 tiles)
+static size_t pass_bitmap_bytes(int w, int h, int p) {
+    const YkPassGeom& g = kGeom[p];
+    return (size_t)((w + g.bw - 1) / g.bw) * ((h + g.bh - 1) / g.bh) * g.bits / 8;
+}
+
+// the box (L, T, R, B) of the tiles pass p accepted, from its counters in the header: the analysis keeps w - L and
+// INT_MAX / 2 - T so that every update is an atomicMax; T stays imgH when the pass accepted no tile
+static void pass_box(const int* hdr, int p, int w, int imgH, int box[4]) {
+    const int* st = hdr + YK_HD_PASS0 + p * YK_ST_STRIDE;
+    box[0] = w - st[YK_ST_MINX]; box[1] = st[YK_ST_MINY] ? INT_MAX / 2 - st[YK_ST_MINY] : imgH;
+    box[2] = st[YK_ST_MAXX]; box[3] = st[YK_ST_MAXY];
+}
+
+// a run of all seven passes, in Convert()'s order
+static void run_all_passes(YkRun& run) { run.nPasses = YK_NPASS; for (int i = 0; i < YK_NPASS; i++) run.passId[i] = i; }
+
 struct YkSlotHost {
     YkSlotDev d;
-    bool haveImage = false, borrowed = false, dirty = true;
+    bool haveImage = false, dirty = true;
     int32_t* owned[4] = { 0, 0, 0, 0 };
     uint8_t* ownedU8[4] = { 0, 0, 0, 0 };     // packed upload: device planes, pinned staging, "staging is free again" event
     uint8_t* stageHost = nullptr; size_t stageBytes = 0;
@@ -54,7 +72,7 @@ struct YkSlotHost {
     size_t arBitmap[YK_NPASS], arRgb[YK_NPASS], arIdx[3], arType[3], arKept = 0;
     int arMask = 0; bool arR2 = false, arHasKept = false;
     // what is valid on the device for the current image
-    bool k1Ran = false;          // r2Seg / latRGB are current
+    bool k1Ran = false;          // a run has been enqueued since the last reset: yk_fetch_all has results to return
     bool alphaRan = false, alphaFetched = false;
     bool prepared = false;       // fused 7-pass cascade results present
     int  preparedReject = 0, nextPass = 0;
@@ -71,14 +89,12 @@ struct YkSlotHost {
     int  chromaHalf[4] = { 0, 0, 0, 0 };
     bool chromaReady = false;
     int  hdr[YK_HD_INTS];        // harvested copy: per-pass stats of the run that produced them, alpha box, R2 totals
-    long long resultBytes[6] = { 0, 0, 0, 0, 0, 0 };
     // alpha results (host)
     int bound[4] = { 0, 0, 0, 0 }, remaining = 0, wroteChunk = 0, chunkBBox[4] = { 0, 0, 0, 0 };
     std::vector<uint8_t> alphaBitmap;
     std::vector<void*> devAllocs;        // every device allocation of the slot (freed by yk_destroy)
-    // strip mode: one allocation [3 * w int32 pixel row][latW touch words from above][latW touch words from below]
+    // strip mode: the halo allocation the neighbours write into (layout: halo_layout)
     uint8_t* haloIn = nullptr; size_t haloBytes = 0;
-    size_t haloFlagsOffset = 0;  // five u32 epoch flags written by the neighbours: see yk_strip_run
     void* peerAbove = nullptr; void* peerBelow = nullptr;     // the neighbours' halo allocations as mapped in this process
     unsigned stripEpoch = 0;
     bool strip = false;          // yk_strip_config placed the current image in a strip set
@@ -249,17 +265,12 @@ static int create_fill(yk_ctx* c) {
     auto supers = [](size_t g) { return (g + YK_SUPER - 1) / YK_SUPER; };
     size_t offTot[YK_NPASS], offSup[YK_NPASS], off = up(YK_HD_INTS * sizeof(int));
     for (int p = 0; p < YK_NPASS; p++) {
-        const YkPassGeom& g = kGeom[p];
-        const size_t nGroups = groups(((W + g.bw - 1) / g.bw) * ((H + g.bh - 1) / g.bh) * (size_t)g.bits / 8);
+        const size_t nGroups = groups(pass_bitmap_bytes(maxW, maxH, p));
         offTot[p] = off; off += up(nGroups * sizeof(uint32_t));
         offSup[p] = off; off += up(supers(nGroups) * sizeof(uint32_t));
     }
-    size_t offNib[YK_NPASS];
-    for (int p = 0; p < YK_NPASS; p++) {
-        const YkPassGeom& g = kGeom[p];
-        offNib[p] = off;
-        off += up(((W + g.bw - 1) / g.bw) * ((H + g.bh - 1) / g.bh) * (size_t)g.bits / 2 + 16);
-    }
+    size_t offNib[YK_NPASS];                 // 4 bits per tile: 4 bytes per bitmap byte
+    for (int p = 0; p < YK_NPASS; p++) { offNib[p] = off; off += up(4 * pass_bitmap_bytes(maxW, maxH, p) + 16); }
     const size_t r2Groups = groups((W / 8) * (H / 8));
     const size_t offR2Tot = off; off += up(r2Groups * sizeof(unsigned long long));
     const size_t offR2Sup = off; off += up(supers(r2Groups) * sizeof(unsigned long long));
@@ -267,11 +278,7 @@ static int create_fill(yk_ctx* c) {
     const size_t offCell = off; off += up((H / 4 + 1) * nbx * sizeof(uint16_t) + 4);
     const size_t offTouch = off; off += up(latW * latH * sizeof(uint32_t));
     size_t offBitmap[YK_NPASS];          // accept bits are OR-ed in by yk_k_analyze: zero before the first pass of an image
-    for (int p = 0; p < YK_NPASS; p++) {
-        const YkPassGeom& g = kGeom[p];
-        offBitmap[p] = off;
-        off += up(((W + g.bw - 1) / g.bw) * ((H + g.bh - 1) / g.bh) * (size_t)g.bits / 8 + 8);
-    }
+    for (int p = 0; p < YK_NPASS; p++) { offBitmap[p] = off; off += up(pass_bitmap_bytes(maxW, maxH, p) + 8); }
     c->zeroStride = off;
     CK(cudaMalloc((void**)&c->zeroArea, c->zeroStride * maxSlots));
     CK(cudaMemsetAsync(c->zeroArea, 0, c->zeroStride * maxSlots, c->stream));     // on the context's own (non-blocking) stream: ordered before its first launch
@@ -380,7 +387,18 @@ extern "C" int yk_profile_read(yk_ctx* c, double ms[8], long long count[8]) {
 }
 
 static int slot_ok(yk_ctx* c, int slot) { return c && slot >= 0 && slot < c->maxSlots; }
-static int upload_slots_fwd(yk_ctx* c, int slot0, int nSlots);
+
+static int upload_slots(yk_ctx* c, int slot0, int nSlots) {
+    for (int i = slot0; i < slot0 + nSlots; i++) {
+        YkSlotHost& s = c->slots[i];
+        if (s.dirty) {
+            if (c->noHostWait) return YK_ERR_STATE;
+            CK(cudaMemcpyAsync(c->slotsDev + i, &s.d, sizeof(YkSlotDev), cudaMemcpyHostToDevice, c->stream));
+            s.dirty = false;
+        }
+    }
+    return YK_OK;
+}
 
 static int configure_slot(yk_ctx* c, int slot, int nPlanes, int w, int h) {
     if (nPlanes < 3 || nPlanes > 4 || w < 4 || h < 4 || (w & 3) || (h & 3)) return YK_ERR_ARG;
@@ -441,7 +459,6 @@ static int use_packed_planes(yk_ctx* c, int slot) {
     }
     s.d.isU8 = 1; s.d.pitchU8 = (s.d.w + 15) / 16 * 16;
     s.int32Valid = false;
-    s.borrowed = false;
     const int rc = encode_slot_tmaps(s);
     if (rc) return rc;
     return yk_reset_state(c, slot);
@@ -486,7 +503,6 @@ extern "C" int yk_set_image(yk_ctx* c, int slot, const int32_t* const* planes, i
     s.d.isU8 = 0; s.d.pitchU8 = 0;
     s.int32Valid = true;
     for (int p = nPlanes; p < 4; p++) { s.d.plane[p] = nullptr; s.d.planeU8[p] = nullptr; }
-    s.borrowed = false;
     if ((rc = encode_slot_tmaps(s))) return rc;
     rc = yk_reset_state(c, slot);
     if (bad & ~255u) s.rangeErr = 1;
@@ -497,7 +513,7 @@ extern "C" int yk_set_image(yk_ctx* c, int slot, const int32_t* const* planes, i
 static int ensure_int32(yk_ctx* c, int slot) {
     YkSlotHost& s = c->slots[slot];
     if (s.int32Valid) return YK_OK;
-    int rc = upload_slots_fwd(c, slot, 1);
+    int rc = upload_slots(c, slot, 1);
     if (rc) return rc;
     yk_launch_expand(c->slotsDev, slot, s.d.nPlanes, s.d.w, s.d.h, s.owned, c->stream);
     c->launches++;
@@ -518,7 +534,6 @@ extern "C" int yk_set_image_device(yk_ctx* c, int slot, const int32_t* const* de
     }
     s.d.isU8 = 0; s.d.pitchU8 = 0; s.int32Valid = true;
     for (int p = nPlanes; p < 4; p++) s.d.plane[p] = nullptr;
-    s.borrowed = true;
     if ((rc = encode_slot_tmaps(s))) return rc;
     return yk_reset_state(c, slot);
 }
@@ -567,20 +582,6 @@ extern "C" int yk_set_image_interleaved_device(yk_ctx* c, int slot, const uint8_
 extern "C" int32_t* yk_device_plane(yk_ctx* c, int slot, int p) {
     if (!slot_ok(c, slot) || p < 0 || p >= c->maxPlanes) return nullptr;
     return c->slots[slot].owned[p];
-}
-
-static int upload_slots(yk_ctx* c, int slot0, int nSlots);
-static int upload_slots_fwd(yk_ctx* c, int slot0, int nSlots) { return upload_slots(c, slot0, nSlots); }
-static int upload_slots(yk_ctx* c, int slot0, int nSlots) {
-    for (int i = slot0; i < slot0 + nSlots; i++) {
-        YkSlotHost& s = c->slots[i];
-        if (s.dirty) {
-            if (c->noHostWait) return YK_ERR_STATE;
-            CK(cudaMemcpyAsync(c->slotsDev + i, &s.d, sizeof(YkSlotDev), cudaMemcpyHostToDevice, c->stream));
-            s.dirty = false;
-        }
-    }
-    return YK_OK;
 }
 
 static int check_batch(yk_ctx* c, int slot0, int nSlots) {
@@ -635,11 +636,8 @@ static int enqueue(yk_ctx* c, int slot0, int nSlots, const YkRun& run, bool doEm
         if (!s.cellsClean) {
             fresh = false;
             // a pass that runs again on a used state starts from an empty bitmap (FittingQuadSmooth allocates pFillBitMap per call, EC.cpp:3770-3777)
-            for (int p = 0; p < run.nPasses; p++) {
-                const YkPassGeom& g = kGeom[run.passId[p]];
-                const size_t nb = (size_t)((s.d.w + g.bw - 1) / g.bw) * ((s.d.h + g.bh - 1) / g.bh) * g.bits / 8;
-                CK(cudaMemsetAsync(s.d.bitmap[run.passId[p]], 0, nb, c->stream));
-            }
+            for (int p = 0; p < run.nPasses; p++)
+                CK(cudaMemsetAsync(s.d.bitmap[run.passId[p]], 0, pass_bitmap_bytes(s.d.w, s.d.h, run.passId[p]), c->stream));
         }
     }
     if ((rc = upload_slots(c, slot0, nSlots))) return rc;
@@ -661,8 +659,7 @@ static int enqueue(yk_ctx* c, int slot0, int nSlots, const YkRun& run, bool doEm
         int gradGroups = 0;
         if (doEmit)
             for (int p = 0; p < krun.nPasses; p++) {
-                const YkPassGeom& g = kGeom[krun.passId[p]];
-                const int nWords = ((a.d.w + g.bw - 1) / g.bw) * ((a.d.h + g.bh - 1) / g.bh) * g.bits / 8;
+                const int nWords = (int)pass_bitmap_bytes(a.d.w, a.d.h, krun.passId[p]);
                 gradGroups += (nWords + YK_EMIT_THREADS - 1) / YK_EMIT_THREADS;
             }
         const int nTiles = (a.d.w / 8) * (a.d.h / 8);
@@ -688,10 +685,10 @@ static int enqueue_r1_fused(yk_ctx* c, int slot, int mode3BitOnly, bool useAlpha
 extern "C" int yk_analyze(yk_ctx* c, int slot0, int nSlots, int stages, int rejectFactor) {
     if (!c || rejectFactor < 0 || rejectFactor > 64) return YK_ERR_ARG;
     if ((stages & YK_STAGE_RANGEDYN) && (stages & YK_STAGE_RANGEDYN3)) return YK_ERR_ARG;
-    YkRun run; memset(&run, 0, sizeof run);
+    YkRun run{};
     run.rejectFactor = rejectFactor;
     run.doAlpha = (stages & YK_STAGE_ALPHA) ? 1 : 0;
-    if (stages & YK_STAGE_GRADIENT) { run.nPasses = YK_NPASS; for (int i = 0; i < YK_NPASS; i++) run.passId[i] = i; }
+    if (stages & YK_STAGE_GRADIENT) run_all_passes(run);
     int rc = check_batch(c, slot0, nSlots);
     if (rc) return rc;
     if (stages & YK_STAGE_GRADIENT)
@@ -718,10 +715,6 @@ extern "C" int yk_prepare_quad_smooth(yk_ctx* c, int slot, int rejectFactor) {
 // ---- results to the host ---------------------------------------------------------------------------------
 // One pinned arena per slot receives every result stream of the last run with two synchronisations (the header with the
 // stream lengths first, then all streams at their actual sizes); the getters then serve from it.
-static size_t pass_bitmap_bytes(const YkSlotHost& s, int p) {
-    const YkPassGeom& g = kGeom[p];
-    return (size_t)((s.d.w + g.bw - 1) / g.bw) * ((s.d.h + g.bh - 1) / g.bh) * g.bits / 8;
-}
 static int harvest(yk_ctx* c, YkSlotHost& s) {
     if (s.harvested) return s.rangeErr ? YK_ERR_RANGE : YK_OK;
     int rc = fetch_hdr(c, s);
@@ -731,7 +724,7 @@ static int harvest(yk_ctx* c, YkSlotHost& s) {
     auto up = [](size_t v) { return (v + 63) / 64 * 64; };
     size_t off = 0;
     for (int p = 0; p < YK_NPASS; p++) {
-        s.arBitmap[p] = off; if (mask & (1 << p)) off += up(pass_bitmap_bytes(s, p));
+        s.arBitmap[p] = off; if (mask & (1 << p)) off += up(pass_bitmap_bytes(s.d.w, s.d.h, p));
         s.arRgb[p] = off; if (mask & (1 << p)) off += up((size_t)s.hdr[YK_HD_PASS0 + p * YK_ST_STRIDE + YK_ST_RGBBYTES]);
     }
     const size_t ni = 16ull * (size_t)s.hdr[YK_HD_R2_CHUNKS], nt = 3ull * (size_t)s.hdr[YK_HD_R2_TILES];
@@ -751,7 +744,7 @@ static int harvest(yk_ctx* c, YkSlotHost& s) {
     }
     for (int p = 0; p < YK_NPASS; p++) {
         if (!(mask & (1 << p))) continue;
-        CK(cudaMemcpyAsync(s.arena + s.arBitmap[p], s.d.bitmap[p], pass_bitmap_bytes(s, p), cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaMemcpyAsync(s.arena + s.arBitmap[p], s.d.bitmap[p], pass_bitmap_bytes(s.d.w, s.d.h, p), cudaMemcpyDeviceToHost, c->stream));
         const size_t nrgb = (size_t)s.hdr[YK_HD_PASS0 + p * YK_ST_STRIDE + YK_ST_RGBBYTES];
         if (nrgb) CK(cudaMemcpyAsync(s.arena + s.arRgb[p], s.d.rgb[p], nrgb, cudaMemcpyDeviceToHost, c->stream));
     }
@@ -768,18 +761,37 @@ static int harvest(yk_ctx* c, YkSlotHost& s) {
 }
 
 // ---- alpha ------------------------------------------------------------------------------------------------
+// MipPrefilter's results (EC.cpp:1287-1403) from the per-tile "kept" bytes ([tilesH][tilesW]) of a w x h image and the box
+// (L, T, R, B) of the kept tiles: the bitmap of the tiles over the box, the pixels that remain, whether a chunk is written
+// and its box in tiles.  A box over the whole image discards the rejection (EC.cpp:1400-1403): no chunk, an empty bitmap,
+// every pixel remains, `kept` is not read and chunkBox is left as it is.  YK_ERR_ARG when the box's tiles leave the grid.
+static int alpha_chunk(const uint8_t* kept, int tilesW, int tilesH, int w, int h, const int box[4],
+                       std::vector<uint8_t>& bitmap, int* remaining, int* wroteChunk, int chunkBox[4]) {
+    const int L = box[0], T = box[1], R = box[2], B = box[3];
+    bitmap.clear();
+    if (yk_box_is_image(box, w, h)) { *remaining = R * B; *wroteChunk = 0; return YK_OK; }
+    const int bx0 = L >> 4, bx1 = (R + 15) >> 4, by0 = T >> 4, by1 = (B + 15) >> 4;
+    const int tWB = bx1 - bx0, tHB = by1 - by0;
+    if (tWB <= 0 || tHB <= 0 || bx1 > tilesW || by1 > tilesH) return YK_ERR_ARG;
+    bitmap.assign((size_t)(tWB * tHB + 7) / 8, 0);
+    int bit = 0, rem = 0;
+    for (int y = 0; y < tHB; y++)
+        for (int x = 0; x < tWB; x++, bit++)
+            if (kept[(size_t)(y + by0) * tilesW + x + bx0]) { bitmap[bit >> 3] |= (uint8_t)(1 << (bit & 7)); rem += 256; }   // EC.cpp:1317-1327
+    *remaining = rem; *wroteChunk = 1;
+    chunkBox[0] = bx0; chunkBox[1] = by0; chunkBox[2] = tWB; chunkBox[3] = tHB;
+    return YK_OK;
+}
+
 static int alpha_finish(yk_ctx* c, YkSlotHost& s) {
     if (s.alphaFetched) return YK_OK;
     int rc = fetch_hdr(c, s);
     if (rc) return rc;
-    const int w = s.d.w, h = s.d.h;
-    const int tw = (w + 15) / 16, th = (h + 15) / 16;
+    const int w = s.d.w, tw = (w + 15) / 16, th = (s.d.h + 15) / 16;
     if (!yk_alpha_box(s.hdr, w, s.bound)) return YK_ERR_ARG;     // fully transparent: outside the reference's domain (sentinel bbox)
-    const int L = s.bound[0], T = s.bound[1], R = s.bound[2], B = s.bound[3];
-    s.alphaBitmap.clear();
-    if (!yk_box_is_image(s.bound, w, s.d.imgH)) {
-        std::vector<uint8_t> keptBuf;
-        const uint8_t* kept;
+    std::vector<uint8_t> keptBuf;
+    const uint8_t* kept = nullptr;
+    if (!yk_box_is_image(s.bound, w, s.d.imgH)) {                 // the kept bytes are only read when the rejection stands
         if (s.harvested && s.arHasKept) kept = s.arena + s.arKept;
         else {
             keptBuf.resize((size_t)tw * th);
@@ -787,19 +799,9 @@ static int alpha_finish(yk_ctx* c, YkSlotHost& s) {
             CK(cudaStreamSynchronize(c->stream));
             kept = keptBuf.data();
         }
-        const int bx0 = L >> 4, bx1 = (R + 15) >> 4, by0 = T >> 4, by1 = (B + 15) >> 4;
-        const int tWB = bx1 - bx0, tHB = by1 - by0;
-        s.alphaBitmap.assign((size_t)(tWB * tHB + 7) / 8, 0);
-        int bit = 0, rem = 0;
-        for (int y = 0; y < tHB; y++)
-            for (int x = 0; x < tWB; x++, bit++)
-                if (kept[(size_t)(y + by0) * tw + x + bx0]) { s.alphaBitmap[bit >> 3] |= (uint8_t)(1 << (bit & 7)); rem += 256; }   // EC.cpp:1317-1327
-        s.remaining = rem; s.wroteChunk = 1;
-        s.chunkBBox[0] = bx0; s.chunkBBox[1] = by0; s.chunkBBox[2] = tWB; s.chunkBBox[3] = tHB;
-        s.d.alphaReset = 0;
-    } else {
-        s.remaining = R * B; s.wroteChunk = 0; s.d.alphaReset = 1;     // EC.cpp:1400-1403
     }
+    if ((rc = alpha_chunk(kept, tw, th, w, s.d.imgH, s.bound, s.alphaBitmap, &s.remaining, &s.wroteChunk, s.chunkBBox))) return rc;
+    s.d.alphaReset = s.wroteChunk ? 0 : 1;
     s.d.alphaValid = 1; s.dirty = true; s.alphaFetched = true;
     return YK_OK;
 }
@@ -812,7 +814,7 @@ extern "C" int yk_alpha_reject(yk_ctx* c, int slot, uint8_t* bitmap, int bitmapC
     if (s.d.nPlanes != 4) return YK_ERR_ARG;
     if (s.d.hasAbove || s.d.hasBelow) return YK_ERR_UNSUPPORTED;    // the alpha bitmap of a strip set is not assembled here
     if (!s.alphaRan) {
-        YkRun run; memset(&run, 0, sizeof run); run.doAlpha = 1; run.rejectFactor = 3;
+        YkRun run{}; run.doAlpha = 1; run.rejectFactor = 3;
         int rc = enqueue(c, slot, 1, run, false, false);
         if (rc) return rc;
     }
@@ -843,14 +845,13 @@ extern "C" int yk_gradient_pass(yk_ctx* c, int slot, int rejectFactor, int shX, 
         // Convert()'s order with the same rejectFactor
         if (pid != s.nextPass || rejectFactor != s.preparedReject) return YK_ERR_STATE;
     } else {
-        YkRun run; memset(&run, 0, sizeof run);
+        YkRun run{};
         run.nPasses = 1; run.passId[0] = pid; run.rejectFactor = rejectFactor;
         if ((rc = enqueue(c, slot, 1, run, true, false))) return rc;
         s.nextPass = -1;
     }
     if ((rc = harvest(c, s))) return rc;
-    const int w = s.d.w;
-    const int nb = (int)pass_bitmap_bytes(s, pid);
+    const int nb = (int)pass_bitmap_bytes(s.d.w, s.d.h, pid);
     const int* st = s.hdr + YK_HD_PASS0 + pid * YK_ST_STRIDE;
     const int nrgb = st[YK_ST_RGBBYTES];
     if (nb > bitmapCap || nrgb > rgbCap) return YK_ERR_CAPACITY;
@@ -860,11 +861,7 @@ extern "C" int yk_gradient_pass(yk_ctx* c, int slot, int rejectFactor, int shX, 
     if (bitmapBytes) *bitmapBytes = nb;
     if (rgbBytes) *rgbBytes = nrgb;
     if (tileDone) *tileDone = st[YK_ST_TILEDONE];
-    if (bbox) {
-        bbox[0] = w - st[YK_ST_MINX];
-        bbox[1] = st[YK_ST_MINY] ? INT_MAX / 2 - st[YK_ST_MINY] : s.d.imgH;
-        bbox[2] = st[YK_ST_MAXX]; bbox[3] = st[YK_ST_MAXY];
-    }
+    if (bbox) pass_box(s.hdr, pid, s.d.w, s.d.imgH, bbox);
     return YK_OK;
 }
 
@@ -877,7 +874,7 @@ extern "C" int yk_range1d(yk_ctx* c, int slot, int plane, uint8_t* idx, int idxC
     if ((s.d.w & 7) || (s.d.h & 7)) return YK_ERR_ARG;          // the reference's own domain (SURVEY.md hazard 11)
     int rc;
     if (!s.r2Valid) {
-        YkRun run; memset(&run, 0, sizeof run); run.rejectFactor = 3;      // no gradient pass: code the unclaimed tiles, scan, gather
+        YkRun run{}; run.rejectFactor = 3;      // no gradient pass: code the unclaimed tiles, scan, gather
         if ((rc = enqueue(c, slot, 1, run, false, true))) return rc;
     }
     if ((rc = harvest(c, s))) return rc;
@@ -1049,6 +1046,20 @@ static int range_dyn_impl(yk_ctx* c, int slot, const int32_t* src, const uint8_t
     return rc;
 }
 
+// one DynamicTileEncode launch of the slot's three colour planes (int32 or packed) as planes of w x ph samples; the caller
+// sets the walk
+static YkR1Launch r1_colour_launch(const YkSlotHost& s, int mode3BitOnly, int ph) {
+    YkR1Launch L;
+    memset(&L, 0, sizeof L);
+    L.nJobs = 3; L.mode3 = mode3BitOnly ? 1 : 0;
+    L.pw = s.d.w; L.ph = ph;
+    for (int p = 0; p < 3; p++) {
+        YkR1Args& a = L.job[p];
+        a.src = s.d.plane[p]; a.srcU8 = s.d.isU8 ? s.d.planeU8[p] : nullptr; a.pitchU8 = s.d.pitchU8; a.out = p;
+    }
+    return L;
+}
+
 // DynamicTileEncode of the three colour planes right behind the analysis, one launch, nothing comes back to the host:
 // the constraint box is derived on the device from the alpha stage's box in the image header
 static int enqueue_r1_fused(yk_ctx* c, int slot, int mode3BitOnly, bool useAlpha) {
@@ -1056,16 +1067,10 @@ static int enqueue_r1_fused(yk_ctx* c, int slot, int mode3BitOnly, bool useAlpha
     const int w = s.d.w, h = s.d.h;
     if ((w & 7) || (h & 7) || w < 32 || h < 32) return YK_ERR_ARG;      // the reference's own domain (SURVEY.md hazard 11)
     if (s.d.hasAbove || s.d.hasBelow) return YK_ERR_UNSUPPORTED;
-    YkR1Launch L;
-    memset(&L, 0, sizeof L);
-    L.nJobs = 3; L.fromHdr = 1; L.useAlpha = useAlpha ? 1 : 0; L.mode3 = mode3BitOnly ? 1 : 0;
-    L.pw = w; L.ph = h;
+    YkR1Launch L = r1_colour_launch(s, mode3BitOnly, h);
+    L.fromHdr = 1; L.useAlpha = useAlpha ? 1 : 0;
     const int full[4] = { 0, 0, w, h };
     L.walk = yk_r1_walk(full, h, 0, 0);                         // the largest possible box: the launch covers it
-    for (int p = 0; p < 3; p++) {
-        YkR1Args& a = L.job[p];
-        a.src = s.d.plane[p]; a.srcU8 = s.d.isU8 ? s.d.planeU8[p] : nullptr; a.pitchU8 = s.d.pitchU8; a.out = p;
-    }
     int rc;
     if ((rc = launch_r1(c, slot, L))) return rc;
     s.r1Fused = mode3BitOnly ? 2 : 1;
@@ -1202,8 +1207,7 @@ extern "C" int yk_result_bytes(yk_ctx* c, int slot, long long out[6]) {
     const int w = s.d.w, h = s.d.h;
     long long bm = 0, rgb = 0;
     for (int p = 0; p < YK_NPASS; p++) {
-        const YkPassGeom& g = kGeom[p];
-        bm += (long long)((w + g.bw - 1) / g.bw) * ((h + g.bh - 1) / g.bh) * g.bits / 8;
+        bm += (long long)pass_bitmap_bytes(w, h, p);
         rgb += s.hdr[YK_HD_PASS0 + p * YK_ST_STRIDE + YK_ST_RGBBYTES];
     }
     out[0] = bm; out[1] = rgb;
@@ -1221,15 +1225,13 @@ extern "C" int yk_fetch_all(yk_ctx* c, int slot, yk_results* out) {
     int rc = harvest(c, s);
     if (rc) return rc;
     memset(out, 0, sizeof *out);
-    const int w = s.d.w;
     for (int p = 0; p < YK_NPASS; p++) {
         if (!(s.arMask & (1 << p))) continue;
         const int* st = s.hdr + YK_HD_PASS0 + p * YK_ST_STRIDE;
-        out->bitmap[p] = s.arena + s.arBitmap[p]; out->bitmapBytes[p] = (int)pass_bitmap_bytes(s, p);
+        out->bitmap[p] = s.arena + s.arBitmap[p]; out->bitmapBytes[p] = (int)pass_bitmap_bytes(s.d.w, s.d.h, p);
         out->rgb[p] = s.arena + s.arRgb[p]; out->rgbBytes[p] = st[YK_ST_RGBBYTES];
         out->tileDone[p] = st[YK_ST_TILEDONE];
-        out->bbox[p][0] = w - st[YK_ST_MINX]; out->bbox[p][1] = st[YK_ST_MINY] ? INT_MAX / 2 - st[YK_ST_MINY] : s.d.imgH;
-        out->bbox[p][2] = st[YK_ST_MAXX]; out->bbox[p][3] = st[YK_ST_MAXY];
+        pass_box(s.hdr, p, s.d.w, s.d.imgH, out->bbox[p]);
     }
     if (s.arR2) {
         out->r2IdxBytes = 16 * s.hdr[YK_HD_R2_CHUNKS]; out->r2TypeBytes = 3 * s.hdr[YK_HD_R2_TILES];
@@ -1248,33 +1250,56 @@ extern "C" int yk_fetch_all(yk_ctx* c, int slot, yk_results* out) {
 }
 
 // ---- multi-GPU: tile-row strips of one large image (SURVEY.md 8e) ----------------------------------------
+// The halo of a strip: one device allocation that its neighbours write into, [pixel row of each colour plane][touch words
+// of the strip above][touch words of the strip below][the epoch flags listed above yk_strip_set_peers].  A strip writes
+// into its neighbours' halos with its own layout, so the layout depends on nothing but the width and the sample type.
+struct YkHaloLayout {
+    size_t planeRowBytes;           // one row of a colour plane: w samples (int32, or bytes after a packed upload)
+    size_t rowStride;               // the row of plane p starts at p * rowStride (planeRowBytes rounded up to 16)
+    size_t pixelRowBytes;           // the three rows
+    size_t touchBytes;              // latW touch words
+    size_t touchTop, touchBottom;   // offsets of the touch words from above / below, 16-byte aligned
+    size_t flags;                   // offset of the epoch flags
+    size_t bytes;                   // size of the allocation
+};
+static YkHaloLayout halo_layout(const YkSlotDev& d) {
+    YkHaloLayout H;
+    H.planeRowBytes = (size_t)d.w * (d.isU8 ? 1 : sizeof(int32_t));
+    H.rowStride = (H.planeRowBytes + 15) / 16 * 16;
+    H.pixelRowBytes = 3 * H.rowStride;
+    H.touchBytes = (size_t)d.latW * sizeof(uint32_t);
+    const size_t touchStride = (H.touchBytes + 15) / 16 * 16;
+    H.touchTop = H.pixelRowBytes;
+    H.touchBottom = H.touchTop + touchStride;
+    H.flags = H.touchBottom + touchStride;
+    H.bytes = H.flags + 64;
+    return H;
+}
+
 extern "C" int yk_strip_config(yk_ctx* c, int slot, int imgH, int y0) {
     if (!slot_ok(c, slot)) return YK_ERR_ARG;
     YkSlotHost& s = c->slots[slot];
     if (!s.haveImage) return YK_ERR_STATE;
-    const int w = s.d.w, h = s.d.h;
+    const int h = s.d.h;
     if (imgH < h || y0 < 0 || y0 + h > imgH || (y0 & 63)) return YK_ERR_ARG;
     if (y0 + h < imgH && (h & 63)) return YK_ERR_ARG;            // only the last strip may end off the 64-row grid
     CK(cudaSetDevice(c->device));
-    const size_t es = s.d.isU8 ? 1 : sizeof(int32_t), rowBytes = ((size_t)w * es + 15) / 16 * 16;
-    const size_t touchBytes = ((size_t)s.d.latW * sizeof(uint32_t) + 15) / 16 * 16;
-    const size_t need = 3 * rowBytes + 2 * touchBytes + 64;
-    if (s.haloBytes < need) {
+    const YkHaloLayout H = halo_layout(s.d);
+    if (s.haloBytes < H.bytes) {
         if (s.haloIn) cudaFree(s.haloIn);
         s.haloIn = nullptr; s.haloBytes = 0;
-        CK(cudaMalloc((void**)&s.haloIn, need));
-        s.haloBytes = need;
+        CK(cudaMalloc((void**)&s.haloIn, H.bytes));
+        s.haloBytes = H.bytes;
     }
     // complete before this returns: the neighbour strips write into this buffer from other streams / processes, and
     // nothing else orders their copies after a clear still queued here
-    CK(cudaMemsetAsync(s.haloIn, 0, need, c->stream));
+    CK(cudaMemsetAsync(s.haloIn, 0, H.bytes, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     s.d.imgH = imgH; s.d.y0 = y0;
     s.d.hasAbove = y0 > 0; s.d.hasBelow = y0 + h < imgH;
-    for (int p = 0; p < 3; p++) s.d.rowBelow[p] = s.d.hasBelow ? (const void*)(s.haloIn + p * rowBytes) : nullptr;
-    s.d.touchInTop = (const uint32_t*)(s.haloIn + 3 * rowBytes);
-    s.d.touchInBottom = (const uint32_t*)(s.haloIn + 3 * rowBytes + touchBytes);
-    s.haloFlagsOffset = 3 * rowBytes + 2 * touchBytes;
+    for (int p = 0; p < 3; p++) s.d.rowBelow[p] = s.d.hasBelow ? (const void*)(s.haloIn + p * H.rowStride) : nullptr;
+    s.d.touchInTop = (const uint32_t*)(s.haloIn + H.touchTop);
+    s.d.touchInBottom = (const uint32_t*)(s.haloIn + H.touchBottom);
     s.stripEpoch = 0; s.peerAbove = nullptr; s.peerBelow = nullptr;
     s.strip = true; s.r1Strip = 0;
     s.dirty = true;
@@ -1285,16 +1310,13 @@ extern "C" int yk_strip_halo_ptrs(yk_ctx* c, int slot, yk_strip_halo* out) {
     if (!slot_ok(c, slot) || !out) return YK_ERR_ARG;
     YkSlotHost& s = c->slots[slot];
     if (!s.haveImage || !s.haloIn) return YK_ERR_STATE;
-    const int w = s.d.w;
+    const YkHaloLayout H = halo_layout(s.d);
     memset(out, 0, sizeof *out);
     out->haloIn = s.haloIn; out->haloBytes = s.haloBytes;
-    const size_t es = s.d.isU8 ? 1 : sizeof(int32_t), rowBytes = ((size_t)w * es + 15) / 16 * 16;
-    out->pixelRowInOffset = 0; out->pixelRowBytes = 3 * rowBytes; out->pixelRowStride = rowBytes;
-    out->touchInTopOffset = out->pixelRowBytes;
-    out->touchBytes = (size_t)s.d.latW * sizeof(uint32_t);
-    out->touchInBottomOffset = (size_t)((const uint8_t*)s.d.touchInBottom - s.haloIn);
+    out->pixelRowInOffset = 0; out->pixelRowBytes = H.pixelRowBytes; out->pixelRowStride = H.rowStride;
+    out->touchInTopOffset = H.touchTop; out->touchInBottomOffset = H.touchBottom; out->touchBytes = H.touchBytes;
     for (int p = 0; p < 3; p++) out->pixelRowOut[p] = s.d.isU8 ? (const void*)s.d.planeU8[p] : (const void*)s.d.plane[p];   // first pixel row of each colour plane
-    out->planeRowBytes = (size_t)w * es;
+    out->planeRowBytes = H.planeRowBytes;
     out->touchOutTop = s.d.touchMap;                                                         // lattice row 0
     out->touchOutBottom = s.d.touchMap + (size_t)(s.d.latH - 1) * s.d.latW;                  // lattice row h/4
     return YK_OK;
@@ -1304,10 +1326,10 @@ extern "C" int yk_strip_phase(yk_ctx* c, int slot, int phase, int rejectFactor) 
     if (!slot_ok(c, slot) || (phase != 0 && phase != 1) || rejectFactor < 0 || rejectFactor > 64) return YK_ERR_ARG;
     YkSlotHost& s = c->slots[slot];
     if (!s.haveImage || !s.haloIn) return YK_ERR_STATE;
-    YkRun run; memset(&run, 0, sizeof run);
+    YkRun run{};
     run.rejectFactor = rejectFactor;
     run.doAlpha = s.d.nPlanes == 4;
-    run.nPasses = YK_NPASS; for (int i = 0; i < YK_NPASS; i++) run.passId[i] = i;
+    run_all_passes(run);
     if (phase == 0) {
         if (s.prepared || s.nextPass || !s.cellsClean) return YK_ERR_STATE;         // needs a fresh state
         return enqueue(c, slot, 1, run, true, true, 1);
@@ -1346,16 +1368,9 @@ static int enqueue_r1_strip(yk_ctx* c, int slot, int mode3BitOnly, const int ima
     if (s.d.alphaValid != maskValid || s.d.alphaReset != maskReset) { s.d.alphaValid = maskValid; s.d.alphaReset = maskReset; s.dirty = true; }
     int rc;
     if ((rc = upload_slots(c, slot, 1))) return rc;
-    YkR1Launch L;
-    memset(&L, 0, sizeof L);
-    L.nJobs = 3; L.mode3 = mode3BitOnly ? 1 : 0;
-    L.pw = w; L.ph = imgH;
+    YkR1Launch L = r1_colour_launch(s, mode3BitOnly, imgH);
     const YkR1Walk g = yk_r1_walk(box, imgH, 0, 0);
     L.walk = yk_r1_window(g, s.d.y0, s.d.h);
-    for (int p = 0; p < 3; p++) {
-        YkR1Args& a = L.job[p];
-        a.src = s.d.plane[p]; a.srcU8 = s.d.isU8 ? s.d.planeU8[p] : nullptr; a.pitchU8 = s.d.pitchU8; a.out = p;
-    }
     s.r1Strip = 0;                                               // the streams are about to be replaced
     if ((rc = launch_r1(c, slot, L))) return rc;
     s.r1Strip = mode3BitOnly ? 2 : 1;
@@ -1378,7 +1393,8 @@ extern "C" int yk_strip_range_dyn(yk_ctx* c, int slot, int mode3BitOnly, const i
 // Every strip enqueues the whole image on its own stream: the two exchanges are device-to-device copies into the
 // neighbours' halo allocations (peer-mapped: NVLink P2P), each followed by a one-thread kernel that publishes an epoch
 // number in the neighbour's halo; before it uses what a neighbour sends, a strip's stream runs a one-thread kernel that
-// waits for that number.  No host barrier, no collective.  Flags (u32, in the strip's own halo, written by neighbours):
+// waits for that number.  No host barrier, no collective.  Flags (u32 at YkHaloLayout::flags in the strip's own halo,
+// written by neighbours):
 //   [0] pixel row of the strip below has landed        [1] touch words of the strip above   [2] touch words of the strip below
 //   [3] the strip above has finished the image         [4] the strip below has finished the image
 extern "C" int yk_strip_set_peers(yk_ctx* c, int slot, void* aboveHalo, void* belowHalo) {
@@ -1426,12 +1442,10 @@ static int strip_run_enqueue(yk_ctx* c, int slot, int rejectFactor, int stages) 
     s.pendingHarvest = false;
     YkNoHostWait guard(c);
     const unsigned e = ++s.stripEpoch;
-    const size_t es = s.d.isU8 ? 1 : sizeof(int32_t), rowBytes = ((size_t)s.d.w * es + 15) / 16 * 16;
-    const size_t touchBytes = (size_t)s.d.latW * sizeof(uint32_t);
-    const size_t offTop = (size_t)((const uint8_t*)s.d.touchInTop - s.haloIn), offBottom = (size_t)((const uint8_t*)s.d.touchInBottom - s.haloIn);
-    unsigned* mine = (unsigned*)(s.haloIn + s.haloFlagsOffset);
-    unsigned* above = s.peerAbove ? (unsigned*)((uint8_t*)s.peerAbove + s.haloFlagsOffset) : nullptr;     // same layout: same width and sample type
-    unsigned* below = s.peerBelow ? (unsigned*)((uint8_t*)s.peerBelow + s.haloFlagsOffset) : nullptr;
+    const YkHaloLayout H = halo_layout(s.d);
+    unsigned* mine = (unsigned*)(s.haloIn + H.flags);
+    unsigned* above = s.peerAbove ? (unsigned*)((uint8_t*)s.peerAbove + H.flags) : nullptr;     // same layout: same width and sample type
+    unsigned* below = s.peerBelow ? (unsigned*)((uint8_t*)s.peerBelow + H.flags) : nullptr;
     // the neighbours have finished the previous image: their halos may be overwritten, and they have read what we sent
     if (e > 1 && (above || below)) { yk_launch_flag_wait(above ? mine + 3 : nullptr, below ? mine + 4 : nullptr, e - 1, c->stream); c->launches++; }
     if ((rc = yk_reset_state(c, slot))) return rc;
@@ -1439,15 +1453,15 @@ static int strip_run_enqueue(yk_ctx* c, int slot, int rejectFactor, int stages) 
     if (above) {
         for (int p = 0; p < 3; p++) {
             const void* src = s.d.isU8 ? (const void*)s.d.planeU8[p] : (const void*)s.d.plane[p];
-            CK(cudaMemcpyAsync((uint8_t*)s.peerAbove + p * rowBytes, src, (size_t)s.d.w * es, cudaMemcpyDefault, c->stream));
+            CK(cudaMemcpyAsync((uint8_t*)s.peerAbove + p * H.rowStride, src, H.planeRowBytes, cudaMemcpyDefault, c->stream));
         }
         yk_launch_flag_set(above + 0, nullptr, e, c->stream); c->launches++;
     }
     if (below) { yk_launch_flag_wait(mine + 0, nullptr, e, c->stream); c->launches++; }
     if ((rc = yk_strip_phase(c, slot, 0, rejectFactor))) return rc;
     // exchange 2: boundary touch words, both directions
-    if (above) CK(cudaMemcpyAsync((uint8_t*)s.peerAbove + offBottom, s.d.touchMap, touchBytes, cudaMemcpyDefault, c->stream));
-    if (below) CK(cudaMemcpyAsync((uint8_t*)s.peerBelow + offTop, s.d.touchMap + (size_t)(s.d.latH - 1) * s.d.latW, touchBytes, cudaMemcpyDefault, c->stream));
+    if (above) CK(cudaMemcpyAsync((uint8_t*)s.peerAbove + H.touchBottom, s.d.touchMap, H.touchBytes, cudaMemcpyDefault, c->stream));
+    if (below) CK(cudaMemcpyAsync((uint8_t*)s.peerBelow + H.touchTop, s.d.touchMap + (size_t)(s.d.latH - 1) * s.d.latW, H.touchBytes, cudaMemcpyDefault, c->stream));
     if (above || below) { yk_launch_flag_set(above ? above + 2 : nullptr, below ? below + 1 : nullptr, e, c->stream); c->launches++; }
     // R1 needs nothing from the neighbours: it runs while their touch words travel
     if ((stages & (YK_STAGE_RANGEDYN | YK_STAGE_RANGEDYN3)) && (rc = enqueue_r1_strip(c, slot, (stages & YK_STAGE_RANGEDYN3) != 0, nullptr))) return rc;
@@ -1525,26 +1539,19 @@ extern "C" int yk_alpha_kept(yk_ctx* c, int slot, uint8_t* kept, int keptCap, in
 extern "C" int yk_alpha_assemble(const uint8_t* kept, int tilesW, int tilesH, int w, int h, const int boundPx[4],
                                  uint8_t* bitmap, int bitmapCap, int* bitmapBytes, int* remainingPixels, int* wroteChunk, int chunkBBoxTiles[4]) {
     if (!kept || !boundPx || tilesW < 1 || tilesH < 1 || !bitmapBytes) return YK_ERR_ARG;
-    const int L = boundPx[0], T = boundPx[1], R = boundPx[2], B = boundPx[3];
     *bitmapBytes = 0;
-    if (L == 0 && T == 0 && R == w && B == h) {                    // EC.cpp:1400-1403: the rejection is discarded
-        if (remainingPixels) *remainingPixels = R * B;
-        if (wroteChunk) *wroteChunk = 0;
-        return YK_OK;
+    std::vector<uint8_t> bm;
+    int rem = 0, wrote = 0, box[4];
+    const int rc = alpha_chunk(kept, tilesW, tilesH, w, h, boundPx, bm, &rem, &wrote, box);
+    if (rc) return rc;
+    if (wrote) {
+        if ((int)bm.size() > bitmapCap || !bitmap) return YK_ERR_CAPACITY;
+        memcpy(bitmap, bm.data(), bm.size());
+        *bitmapBytes = (int)bm.size();
+        if (chunkBBoxTiles) memcpy(chunkBBoxTiles, box, sizeof box);
     }
-    const int bx0 = L >> 4, bx1 = (R + 15) >> 4, by0 = T >> 4, by1 = (B + 15) >> 4;
-    const int tWB = bx1 - bx0, tHB = by1 - by0, nb = (tWB * tHB + 7) / 8;
-    if (tWB <= 0 || tHB <= 0 || bx1 > tilesW || by1 > tilesH) return YK_ERR_ARG;
-    if (nb > bitmapCap || !bitmap) return YK_ERR_CAPACITY;
-    memset(bitmap, 0, (size_t)nb);
-    int bit = 0, rem = 0;
-    for (int y = 0; y < tHB; y++)
-        for (int x = 0; x < tWB; x++, bit++)
-            if (kept[(size_t)(y + by0) * tilesW + x + bx0]) { bitmap[bit >> 3] |= (uint8_t)(1 << (bit & 7)); rem += 256; }   // EC.cpp:1317-1327
-    *bitmapBytes = nb;
     if (remainingPixels) *remainingPixels = rem;
-    if (wroteChunk) *wroteChunk = 1;
-    if (chunkBBoxTiles) { chunkBBoxTiles[0] = bx0; chunkBBoxTiles[1] = by0; chunkBBoxTiles[2] = tWB; chunkBBoxTiles[3] = tHB; }
+    if (wroteChunk) *wroteChunk = wrote;
     return YK_OK;
 }
 
