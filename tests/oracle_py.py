@@ -85,8 +85,8 @@ class Oracle:
         assert rc == 0
         return dict(bitmap=bm[:nb.value].copy(), rgb=rgb[:nr.value].copy(), bbox=list(bbox), tiledone=done.value)
 
-    def gradient_cascade(self):
-        return [self.gradient_pass(sx, sy) for sx, sy in PASS_ORDER]
+    def gradient_cascade(self, reject=3):
+        return [self.gradient_pass(sx, sy, reject=reject) for sx, sy in PASS_ORDER]
 
     def range1d(self, plane, want_debug=False):
         idx = np.zeros(self.w * self.h + 8, np.uint8)

@@ -34,25 +34,44 @@ def results_digest(r) -> str:
     return h.hexdigest()
 
 
-def check_image(ctx: "capi.Context", planes: np.ndarray, stages, *, fused=True, state=True, slot=0, load=None):
-    """stages as in tests/cases.py.  fused=True: one yk_analyze then getters; False: stage-by-stage calls.
-    load(ctx, planes, slot): how the samples get into the context (default: yk_set_image from host planes)."""
+def fused_stages(planes: np.ndarray, stages) -> int:
+    """The yk_analyze stage flags that run `stages` (as in tests/cases.py) in one call: R1 only inside its domain
+    (multiples of 8, at least 32 x 32), alpha only on four planes."""
     c, h, w = planes.shape
-    o = Oracle(planes)
+    st = ((capi.STAGE_ALPHA if "alpha" in stages and c == 4 else 0) | (capi.STAGE_GRADIENT if "grad" in stages else 0)
+          | (capi.STAGE_RANGE1D if "r2" in stages else 0))
+    if ("r1" in stages or "r1_3bit" in stages) and w >= 32 and h >= 32 and w % 8 == 0 and h % 8 == 0:
+        st |= capi.STAGE_RANGEDYN3 if "r1_3bit" in stages else capi.STAGE_RANGEDYN
+    return st
+
+
+def check_image(ctx: "capi.Context", planes: np.ndarray, stages, *, fused=True, state=True, slot=0, load=None, reject=3):
+    """stages as in tests/cases.py.  fused=True: one yk_analyze then getters; False: stage-by-stage calls.
+    load(ctx, planes, slot): how the samples get into the context (default: yk_set_image from host planes).
+    reject: the rejectFactor of the gradient stage (0..64), passed to yk_analyze, yk_gradient_pass and the oracle."""
     if load is None:
         ctx.set_image(planes, slot)
     else:
         load(ctx, planes, slot)
+    st = fused_stages(planes, stages)
+    if fused:
+        ctx.analyze(st, slot0=slot, reject=reject)
+    check_results(ctx, planes, stages, slot=slot, state=state, reject=reject,
+                  r1_fused=fused and bool(st & (capi.STAGE_RANGEDYN | capi.STAGE_RANGEDYN3)))
+
+
+def check_results(ctx: "capi.Context", planes: np.ndarray, stages, *, slot=0, state=True, reject=3, r1_fused=False, r1_without_dst=False,
+                  r1_dst=True):
+    """The results of `stages` in `slot` against the oracle, once the image is loaded: whatever yk_analyze left there, and
+    the getters run the stages it did not (stage by stage).  r1_fused: yk_analyze coded R1, its streams are fetched as they
+    are first; r1_without_dst: R1 is also fetched once without a write-back plane when it was not fused; r1_dst: then
+    each plane is coded again with the write-back plane (this replaces the fused streams)."""
+    c, h, w = planes.shape
+    o = Oracle(planes)
     do_alpha = "alpha" in stages and c == 4
     do_grad = "grad" in stages
     do_r2 = "r2" in stages
     do_r1 = "r1" in stages or "r1_3bit" in stages
-    r1_fused = fused and do_r1 and w >= 32 and h >= 32 and w % 8 == 0 and h % 8 == 0
-    if fused:
-        st = (capi.STAGE_ALPHA if do_alpha else 0) | (capi.STAGE_GRADIENT if do_grad else 0) | (capi.STAGE_RANGE1D if do_r2 else 0)
-        if r1_fused:        # DynamicTileEncode of R, G, B in the same call (one launch behind the analysis)
-            st |= capi.STAGE_RANGEDYN3 if "r1_3bit" in stages else capi.STAGE_RANGEDYN
-        ctx.analyze(st, slot0=slot)
     if do_alpha:
         want = o.alpha()
         if want is not None:
@@ -64,8 +83,8 @@ def check_image(ctx: "capi.Context", planes: np.ndarray, stages, *, fused=True, 
             _eq(got["bitmap"], want["bitmap"], "alpha bitmap")
     if do_grad:
         for k, (sx, sy) in enumerate(PASS_ORDER):
-            want = o.gradient_pass(sx, sy)
-            got = ctx.gradient_pass(sx, sy, slot)
+            want = o.gradient_pass(sx, sy, reject=reject)
+            got = ctx.gradient_pass(sx, sy, slot, reject=reject)
             assert got["tiledone"] == want["tiledone"], (f"pass {k} tileDone", got["tiledone"], want["tiledone"])
             _eq(got["bitmap"], want["bitmap"], f"pass {k} bitmap")
             assert got["bbox"] == want["bbox"], (f"pass {k} bbox", got["bbox"], want["bbox"])
@@ -86,14 +105,15 @@ def check_image(ctx: "capi.Context", planes: np.ndarray, stages, *, fused=True, 
             _eq(s["recon"][n].ravel(), o.state(8 + n), f"recon{n}")
     if do_r1:
         wants = [o.range_dyn(n, mode3="r1_3bit" in stages, want_dst=True) for n in range(3)]
-        if r1_fused:        # the streams yk_analyze left on the device
+        if r1_fused or r1_without_dst:        # the streams yk_analyze left on the device / coded without a write-back plane
+            what = "fused R1" if r1_fused else "R1 without dst"
             for n in range(3):
                 got = ctx.range_dyn(n, mode3="r1_3bit" in stages, slot=slot, want_dst=False)
                 assert got["constraint"] == wants[n]["constraint"]
-                _eq(got["defs"], wants[n]["defs"], f"fused R1 defs plane {n}")
+                _eq(got["defs"], wants[n]["defs"], f"{what} defs plane {n}")
                 assert got["n_nibbles"] == wants[n]["n_nibbles"]
-                _eq(got["nibbles"], wants[n]["nibbles"], f"fused R1 nibbles plane {n}")
-        for n in range(3):
+                _eq(got["nibbles"], wants[n]["nibbles"], f"{what} nibbles plane {n}")
+        for n in range(3 if r1_dst else 0):
             want = wants[n]
             got = ctx.range_dyn(n, mode3="r1_3bit" in stages, slot=slot, want_dst=True)
             assert got["constraint"] == want["constraint"]
@@ -104,11 +124,15 @@ def check_image(ctx: "capi.Context", planes: np.ndarray, stages, *, fused=True, 
     o.close()
 
 
-def check_chroma(ctx: "capi.Context", planes: np.ndarray, pre, cfg, modes, slot=0):
-    """The chroma front-end (yk_chroma_prepare + yk_range_dyn_chroma x3) after the stages in `pre`, against the oracle."""
+def check_chroma(ctx: "capi.Context", planes: np.ndarray, pre, cfg, modes, slot=0, load=None):
+    """The chroma front-end (yk_chroma_prepare + yk_range_dyn_chroma x3) after the stages in `pre`, against the oracle.
+    load: as in check_image."""
     c, h, w = planes.shape
     o = Oracle(planes)
-    ctx.set_image(planes, slot)
+    if load is None:
+        ctx.set_image(planes, slot)
+    else:
+        load(ctx, planes, slot)
     st = (capi.STAGE_ALPHA if ("alpha" in pre and c == 4) else 0) | (capi.STAGE_GRADIENT if "grad" in pre else 0)
     if st:
         ctx.analyze(st, slot0=slot)
